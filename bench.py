@@ -2,6 +2,7 @@
 """bench.py -- latent hash-grid fwd+bwd throughput (BASELINE.json metric) on N B200s.
 
     python bench.py --gpus N --steps K --warmup W            # this package (CUDA, C-ABI)
+    python bench.py --steps K --dump-outputs DIR             # + what the last timed step computes, DIR/<name>.npy
     python bench.py --impl reference --steps K --warmup W    # the reference's path on the host cores
     python bench.py --impl reference-gpu                     # the reference's own CUDA kernels (oracle/_ref)
 
@@ -35,6 +36,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 H, W = 512, 768
 NUM_LODS, BITWIDTH, MIN_RES, MAX_RES = 16, 16, 16, 512
@@ -234,7 +236,15 @@ def main():
     ap.add_argument("--no-fit", action="store_true", help="skip the short Kodak-shape fit (fits/hour, second half of the metric)")
     ap.add_argument("--no-nerf", action="store_true", help="skip the NeRF-shape ray-batch data-parallel step (cfg4)")
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip timing the reference's own CUDA kernels (oracle/_ref)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computes (rank 0): feature rows, latent gradient and the "
+                         "shared decoder's scale / shift gradients, as DIR/<name>.npy in float32; the seeded inputs "
+                         "are the same in every run, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours only")
     if args.impl == "reference":
         return reference_arm(args)
     if args.impl == "reference-gpu":
@@ -368,6 +378,18 @@ def main():
         if world > 1:
             dist.barrier()
         total_ms = start.elapsed_time(stop)
+        outputs = None
+        if args.dump_outputs and rank == 0:
+            # The decoder gradients are accumulated into across steps (the timed loop never clears them), so the last
+            # timed step runs once more, untimed, from zeroed ones. One shared decoder: only the sum over the L rows is
+            # defined, and that sum is what a caller receives (grid_ops.LatentHashGrid.backward).
+            gA.zero_()
+            gS.zero_()
+            step(steps - 1, st0)
+            stream.synchronize()
+            last = sets[(steps - 1) % ROTATE]
+            outputs = {"feats": last["feats"].clone(), "grad_latents": last["gl"].clone(),
+                       "grad_A": gA.sum(0, keepdim=True), "grad_shift": gS.sum(0, keepdim=True)}
         # per-kernel launch durations, measured live with CUDA events over K back-to-back launches each
         def timed(fn, graph):
             run(fn, steps, graph)
@@ -658,6 +680,10 @@ def main():
                                 "sample": "3 steps x full %d-point batch (fwd+bwd incl. table decode) after 1 warm-up; "
                                           "OpenMP oracle port of the reference kernels" % n,
                                 "host_cpus": os.cpu_count()}
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy())
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -16,7 +16,7 @@ Restates, operation by operation and in the reference's order:
                                  uniform draws passed in; pinned by tests/golden/sga_ref.npz (make_golden_sga.py)
 
 Pinned against the reference's own Python modules imported under stubs: tests/golden/make_golden.py
-writes tests/golden/latent_ref.npz, tests/test_oracle_golden.py compares.
+writes tests/golden/latent_ref_<case>.npz, tests/test_oracle_golden.py compares.
 """
 import numpy as np
 import torch

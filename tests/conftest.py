@@ -1,3 +1,4 @@
+import glob
 import os
 import sys
 
@@ -29,8 +30,12 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def golden():
-    path = os.path.join(ROOT, "tests", "golden", "latent_ref.npz")
-    return np.load(path)
+    """Every case of tests/golden/latent_ref_<case>.npz (one file per case keeps each under 1 MB), keys '<case>/...'."""
+    out = {}
+    for path in sorted(glob.glob(os.path.join(ROOT, "tests", "golden", "latent_ref_*.npz"))):
+        with np.load(path) as g:
+            out.update({k: g[k] for k in g.files})
+    return out
 
 
 @pytest.fixture(scope="session")

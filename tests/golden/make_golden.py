@@ -1,4 +1,4 @@
-"""Generate tests/golden/latent_ref.npz by running the REFERENCE's own Python modules
+"""Generate tests/golden/latent_ref_<case>.npz (one file per case) by running the REFERENCE's own Python modules
 (imported from /root/reference with its missing third-party deps stubbed) on seeded inputs.
 
 Run in the build container only (`python tests/golden/make_golden.py`); the fixture is
@@ -167,10 +167,10 @@ def main():
         ld2, cb2 = grid.size(use_torchac=False, use_prob_model=True)
         out[p + "size"] = np.array([ld, cb, ld2, cb2], dtype=np.float64)
         cases.append(name)
-    out["cases"] = np.array(cases)
-    path = os.path.join(ROOT, "tests", "golden", "latent_ref.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes;", cases)
+    for name in cases:  # one file per case: each stays under 1 MB
+        path = os.path.join(ROOT, "tests", "golden", "latent_ref_%s.npz" % name)
+        np.savez_compressed(path, **{k: v for k, v in out.items() if k.startswith(name + "/")})
+        print("wrote", path, os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

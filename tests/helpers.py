@@ -9,7 +9,7 @@ def case_from_golden(golden, name):
     p = name + "/"
     dim, L, bw, C, F, layers, hier, dft = [int(v) for v in golden[p + "meta"]]
     d = dict(name=name, dim=dim, L=L, bw=bw, C=C, F=F, layers=layers, hier=bool(hier), dft=bool(dft))
-    for k in golden.files:
+    for k in golden:
         if k.startswith(p):
             d[k[len(p):]] = golden[k]
     d["resolutions"] = [int(v) for v in d["resolutions"]]
@@ -45,6 +45,33 @@ def prob_params_from_case(c):
             packed[fi, 2] = a.reshape(-1)
         d["f%d" % (fi + 1)] = (torch.from_numpy(h), torch.from_numpy(b), torch.from_numpy(a) if a is not None else None)
     return packed, d
+
+
+REF_KERNEL_CASES = {"2d_cfg1": "uniform", "2d_cfg2_arbitrary": "arbitrary", "2d_q4_dense": "uniform",
+                    "3d_cfg4": "arbitrary", "3d_lego24_f4": "uniform"}
+
+
+def ref_kernel_case(g, name):
+    """One case of tests/golden/hashgrid_ref_kernels.npz (outputs of the reference's own CUDA kernels, captured by
+    make_golden_gpu.py) with its seeded table / upstream gradient regenerated: the same draws as make_case(seed=...)
+    there (the coordinate kind decides the first draw; the stored coordinates carry the edge rows)."""
+    p = name + "/"
+    dim, L, bw, F = [int(v) for v in g[p + "meta"]]
+    res = [int(v) for v in g[p + "resolutions"]]
+    coords = g[p + "coords"]
+    n = coords.shape[0]
+    rng = np.random.default_rng(int(g[p + "seed"][0]))
+    if REF_KERNEL_CASES[name] == "uniform":
+        rng.random((n, dim), dtype=np.float32)
+    else:
+        rng.standard_normal((n, dim))
+    sizes, first, T = oracle.level_layout(res, bw, dim)
+    table = rng.standard_normal((T, F)).astype(np.float32)
+    gout = rng.standard_normal((n, L * F)).astype(np.float32)
+    assert np.array_equal(table[:16], g[p + "table_seed_check"])
+    return dict(dim=dim, L=L, bw=bw, F=F, resolutions=res, first_idx=first, T=T, coords=coords, table=table,
+                grad_out=gout, feats=g[p + "feats"], grad_rows=g[p + "grad_rows"], grad_vals=g[p + "grad_vals"],
+                grad_nonzero_rows=int(g[p + "grad_nonzero_rows"][0]), grad_total=g[p + "grad_total"])
 
 
 def rel_err(a, b):

@@ -89,7 +89,7 @@ def test_reference_autograd_functions_over_the_shim_fp32_and_autocast(lib, dim):
 def test_latent_call_pattern_of_the_reference_grid(lib, golden, name):
     """LatentGrid.interpolate of the reference (latent_grid.py:359-370) on top of the shim: decode the table with torch,
     pad a one-channel table to two (repeat(1, 2)), interpolate, take every other column -- against the features and
-    table gradients the reference produced (tests/golden/latent_ref.npz)."""
+    table gradients the reference produced (tests/golden/latent_ref_<case>.npz)."""
     from shacira_b200 import compat
     C = compat.install_as_wisp_C()
     Fn3, Fn2 = _reference_functions(C.ops)

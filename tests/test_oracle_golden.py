@@ -8,7 +8,7 @@ import torch
 
 import oracle
 from oracle import latent_oracle as lo
-from helpers import affine_from_case, case_from_golden, prob_params_from_case, rel_err
+from helpers import REF_KERNEL_CASES, affine_from_case, case_from_golden, prob_params_from_case, ref_kernel_case, rel_err
 
 CASES = ["img_c1f1", "img_c2f4_h", "nerf_c1f4", "nerf_c4f4_dft"]
 
@@ -149,42 +149,17 @@ def _ref_kernel_cases():
     return np.load(path)
 
 
-@pytest.mark.parametrize("name", ["2d_cfg1", "2d_cfg2_arbitrary", "2d_q4_dense", "3d_cfg4", "3d_lego24_f4"])
+@pytest.mark.parametrize("name", list(REF_KERNEL_CASES))
 def test_oracle_matches_reference_cuda_kernels(name):
     """tests/golden/make_golden_gpu.py ran oracle/_ref (the reference's .cu files, unmodified, sm_100a) on a B200.
     Forward: the oracle reproduces the kernel's floats bit for bit. Backward: atomics are order dependent -> 1e-5."""
-    from helpers import rel_err
-    g = _ref_kernel_cases()
-    p = name + "/"
-    dim, L, bw, F = [int(v) for v in g[p + "meta"]]
-    res = [int(v) for v in g[p + "resolutions"]]
-    coords = g[p + "coords"]
-    # regenerate the seeded table / upstream gradient exactly as the capture script did
-    sizes, first, T = oracle.level_layout(res, bw, dim)
-    table, gout = _regen(dim, L, bw, res, coords.shape[0], F, int(g[p + "seed"][0]), name)
-    assert np.array_equal(table[:16], g[p + "table_seed_check"])
-    feats = oracle.forward(coords, table, first, res, bw)
-    assert np.array_equal(feats.view(np.uint32), g[p + "feats"].view(np.uint32))
-    grad = oracle.backward(coords, gout, T, first, res, bw, F)
-    rows = g[p + "grad_rows"]
-    assert rel_err(grad[rows], g[p + "grad_vals"]) <= 1e-5
-    assert int((np.abs(grad).sum(1) != 0).sum()) == int(g[p + "grad_nonzero_rows"][0])
-    assert rel_err(grad.astype(np.float64).sum(0), g[p + "grad_total"]) <= 1e-5
-
-
-def _regen(dim, L, bw, res, n, F, seed, name):
-    """Same draws as helpers.make_case(seed=...) in make_golden_gpu.py (coords kind decides the first draw)."""
-    kinds = {"2d_cfg1": "uniform", "2d_cfg2_arbitrary": "arbitrary", "2d_q4_dense": "uniform", "3d_cfg4": "arbitrary",
-             "3d_lego24_f4": "uniform"}
-    rng = np.random.default_rng(seed)
-    if kinds[name] == "uniform":
-        rng.random((n, dim), dtype=np.float32)
-    else:
-        rng.standard_normal((n, dim))
-    sizes, first, T = oracle.level_layout(res, bw, dim)
-    table = rng.standard_normal((T, F)).astype(np.float32)
-    gout = rng.standard_normal((n, L * F)).astype(np.float32)
-    return table, gout
+    c = ref_kernel_case(_ref_kernel_cases(), name)
+    feats = oracle.forward(c["coords"], c["table"], c["first_idx"], c["resolutions"], c["bw"])
+    assert np.array_equal(feats.view(np.uint32), c["feats"].view(np.uint32))
+    grad = oracle.backward(c["coords"], c["grad_out"], c["T"], c["first_idx"], c["resolutions"], c["bw"], c["F"])
+    assert rel_err(grad[c["grad_rows"]], c["grad_vals"]) <= 1e-5
+    assert int((np.abs(grad).sum(1) != 0).sum()) == c["grad_nonzero_rows"]
+    assert rel_err(grad.astype(np.float64).sum(0), c["grad_total"]) <= 1e-5
 
 
 def test_render_oracle_closed_forms():
