@@ -272,6 +272,20 @@ int shacira_fit_tile_step(const shacira_plan_t* plan, const float* latents, cons
                           int64_t table_rows, float* grad_latents, float* grad_A, float* grad_shift, void* mlp_out,
                           shacira_stream_t stream);
 
+/* The forward-only sibling of shacira_fit_tile_step: turns a model of that shape into pixels (the final PSNR of a fit,
+ * a decoded codec model, a render at another resolution) without writing the [n, 16] feature rows. Reference:
+ * mlp(grid.interpolate(coords)) with STE rounding (latent_grid.py:340-382, nefs/image.py:109-120,152). Same shapes as
+ * shacira_fit_tile_step; the latents are always rounded. `plan`: 2D, any mode; rows of `rgb` [n, 3] and `target` [n, 3]
+ * follow the plan's convention (original point index, or tile order on a sorted-I/O plan). With target != NULL,
+ * *sse_u8 (cleared by the call) receives sum (q(rgb) - q(target))^2 over all n x 3 values with
+ * q(v) = (uint8)(clamp(v, 0, 1) * 255) -- the integer SSE behind the clamped PSNR of wisp/ops/image/metrics.py:39-57;
+ * rgb may then be NULL (PSNR without writing the image). */
+int shacira_fit_render(const shacira_plan_t* plan, const float* latents, const int32_t* first_idx,
+                       const int32_t* resolutions, int32_t num_lods, int32_t codebook_bitwidth, const float* A,
+                       const float* shift, const float* W1, const float* b1, const float* W2, const float* b2,
+                       const float* W3, const float* b3, float* rgb, const float* target, uint64_t* sse_u8,
+                       shacira_stream_t stream);
+
 /* ---- fused Adam over the latent table (SURVEY section 8, row f-4) ------------------------ */
 /* torch.optim.Adam semantics (L2 weight decay added to the gradient, bias correction, eps outside the sqrt) for
  * ONE float32 tensor in place; `step` is a device float counter (starts at 0) that the call advances, so the
@@ -458,6 +472,36 @@ int shacira_fit_optimizer_step(const shacira_adam_seg_t* segs, int32_t num_segs,
                                const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step, double* bits,
                                float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes, uint32_t* ticket,
                                shacira_stream_t stream);
+
+/* Best-state selection inside that launch (the reference's ImageTrainer keeps the state of the lowest rgb_loss and
+ * reports PSNR / bpp from it, image_trainer.py:173-178,305-310,471-502). Every CTA evaluates
+ * loss_t = (float)(*sse / count) -- the SSE the fit kernel wrote for this step's parameters, count = n x 3 -- and, when
+ * loss_t < *best_loss (strict: the first minimum wins, NaN never), stores the PRE-update values of the parameters it
+ * owns: the latent table into `table`, segment i's param into seg_param[i] (NULL: not stored), div [latent_dim] and
+ * A [latent_dim * feature_dim] (the A this step's forward used) by the CTA of the `scale` segment. Only the last CTA
+ * writes *best_loss / *best_step (the step index: *step_small before the call advances it), after every CTA has
+ * evaluated the predicate. Initialise *best_loss to +inf. */
+typedef struct {
+    const double* sse;
+    int64_t count;
+    float* best_loss;
+    int64_t* best_step;
+    float* table;
+    float* seg_param[SHACIRA_MAX_ADAM_SEGS];
+    float* div;
+    float* A;
+} shacira_fit_snapshot_t;
+/* shacira_fit_optimizer_step with the snapshot above (snap != NULL). */
+int shacira_fit_optimizer_step_best(const shacira_adam_seg_t* segs, int32_t num_segs, float* table, float* grad,
+                                    const float* grad_mul, const float* grad2, const float* scale2, float scale2_mul,
+                                    float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float weight_decay,
+                                    float beta1, float beta2, float eps, float* step_small, float* step_table,
+                                    const float* scale, const float* div, float* A_out, int32_t latent_dim,
+                                    int32_t feature_dim, const float* temperature, int32_t diff_sampling, uint64_t seed,
+                                    uint64_t* rng_step, float* w_hat, float* dw, const float* ent_params,
+                                    int32_t ent_layers, const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step,
+                                    double* bits, float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes,
+                                    uint32_t* ticket, const shacira_fit_snapshot_t* snap, shacira_stream_t stream);
 
 /* ---- exchange step of the ray-batch data-parallel path over NVLink / NVSwitch peer memory (SURVEY 8e) ------------
  * north_star: "NeRF ray batches are data-parallel, with the hash-table/latent gradient allreduced ... over NVLink".

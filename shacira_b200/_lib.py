@@ -36,6 +36,12 @@ class AdamSeg(ctypes.Structure):
 
 MAX_ADAM_SEGS = 32
 
+
+class FitSnapshot(ctypes.Structure):
+    """shacira_fit_snapshot_t (include/shacira_b200.h)."""
+    _fields_ = [("sse", _vp), ("count", _i64), ("best_loss", _vp), ("best_step", _vp), ("table", _vp),
+                ("seg_param", _vp * MAX_ADAM_SEGS), ("div", _vp), ("A", _vp)]
+
 # name -> (restype, argtypes); mirrors include/shacira_b200.h one to one.
 SIGNATURES = {
     "shacira_abi_version": (ctypes.c_int, []),
@@ -68,6 +74,7 @@ SIGNATURES = {
     "shacira_mlp_mse_step": (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "shacira_mlp_mse_step_bounded": (ctypes.c_int, [_vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "shacira_fit_tile_step": (ctypes.c_int, [_vp, _vp, _c_int32_p, _c_int32_p, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "shacira_fit_render": (ctypes.c_int, [_vp, _vp, _c_int32_p, _c_int32_p, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "shacira_peer_flags_offset": (_i64, [_i64]),
     "shacira_peer_alloc": (ctypes.c_int, [_i64, ctypes.POINTER(_vp)]),
     "shacira_peer_free": (ctypes.c_int, [_vp]),
@@ -80,6 +87,7 @@ SIGNATURES = {
     "shacira_peer_allreduce_multimem": (ctypes.c_int, [_vp, ctypes.POINTER(_vp), _i64, _i32, _i32, _i64, _vp]),
     "shacira_peer_allreduce_adam": (ctypes.c_int, [ctypes.POINTER(_vp), _i64, _i32, _i32, _i64, ctypes.POINTER(_vp), _i64, _vp, _vp, _vp, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp]),
     "shacira_fit_optimizer_step": (ctypes.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _i32, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i32, _vp, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i64, _vp, _vp]),
+    "shacira_fit_optimizer_step_best": (ctypes.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _i32, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i32, _vp, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "shacira_adam_step": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _i32, _vp]),
     "shacira_adam_step_sum": (ctypes.c_int, [_vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _i32, _i32, _vp]),
     "shacira_adam_step_sum_mul": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _i32, _i32, _vp]),

@@ -631,16 +631,21 @@ int shacira_sga_quantize(const float* latents, const float* uniforms, int64_t co
     return SHACIRA_OK;
 }
 
-int shacira_fit_optimizer_step(const shacira_adam_seg_t* segs, int32_t num_segs, float* table, float* grad,
-                               const float* grad_mul, const float* grad2, const float* scale2, float scale2_mul,
-                               float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float weight_decay, float beta1,
-                               float beta2, float eps, float* step_small, float* step_table, const float* scale,
-                               const float* div, float* A_out, int32_t latent_dim, int32_t feature_dim,
-                               const float* temperature, int32_t diff_sampling, uint64_t seed, uint64_t* rng_step,
-                               float* w_hat, float* dw, const float* ent_params, int32_t ent_layers,
-                               const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step, double* bits,
-                               float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes, uint32_t* ticket,
-                               shacira_stream_t stream) {
+}  // extern "C"
+
+namespace {
+
+// shacira_fit_optimizer_step and its best-state form (snap != NULL): one validation, one launch
+int fit_optimizer_launch(const shacira_adam_seg_t* segs, int32_t num_segs, float* table, float* grad,
+                         const float* grad_mul, const float* grad2, const float* scale2, float scale2_mul,
+                         float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float weight_decay, float beta1,
+                         float beta2, float eps, float* step_small, float* step_table, const float* scale,
+                         const float* div, float* A_out, int32_t latent_dim, int32_t feature_dim,
+                         const float* temperature, int32_t diff_sampling, uint64_t seed, uint64_t* rng_step,
+                         float* w_hat, float* dw, const float* ent_params, int32_t ent_layers,
+                         const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step, double* bits,
+                         float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes, uint32_t* ticket,
+                         const shacira_fit_snapshot_t* snap, shacira_stream_t stream) {
     if (!step_small || !step_table || !ticket || num_segs < 0 || (num_segs > 0 && !segs))
         return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step: NULL argument");
     if (num_segs > SHACIRA_MAX_ADAM_SEGS)
@@ -680,11 +685,63 @@ int shacira_fit_optimizer_step(const shacira_adam_seg_t* segs, int32_t num_segs,
         Tb.ent_rng_step = (unsigned long long*)ent_rng_step; Tb.ent_partials = (float*)ent_scratch; Tb.bits = bits;
         Tb.g_prob = grad_ent_params;
     }
+    shacira_fit_snapshot_t sn;
+    memset(&sn, 0, sizeof(sn));
+    if (snap) {
+        if (!snap->sse || snap->count <= 0 || !snap->best_loss || !snap->best_step || !snap->table)
+            return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_best: snapshot sse / count / best / table missing");
+        if (!A_out || !snap->div || !snap->A)
+            return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_best: the snapshot of div and A needs A_out, div and A");
+        sn = *snap;
+    }
     const int64_t blocks = num_segs + (n + 1023) / 1024;
-    fit_optimizer_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(S, Tb, beta1, beta2, eps, step_small, step_table,
-                                                                         scale, div, A_out, latent_dim, feature_dim, ticket);
+    if (snap)
+        fit_optimizer_kernel<true><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
+            S, Tb, beta1, beta2, eps, step_small, step_table, scale, div, A_out, latent_dim, feature_dim, ticket, sn);
+    else
+        fit_optimizer_kernel<false><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
+            S, Tb, beta1, beta2, eps, step_small, step_table, scale, div, A_out, latent_dim, feature_dim, ticket, sn);
     LAUNCHED();
     return SHACIRA_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int shacira_fit_optimizer_step(const shacira_adam_seg_t* segs, int32_t num_segs, float* table, float* grad,
+                               const float* grad_mul, const float* grad2, const float* scale2, float scale2_mul,
+                               float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float weight_decay, float beta1,
+                               float beta2, float eps, float* step_small, float* step_table, const float* scale,
+                               const float* div, float* A_out, int32_t latent_dim, int32_t feature_dim,
+                               const float* temperature, int32_t diff_sampling, uint64_t seed, uint64_t* rng_step,
+                               float* w_hat, float* dw, const float* ent_params, int32_t ent_layers,
+                               const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step, double* bits,
+                               float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes, uint32_t* ticket,
+                               shacira_stream_t stream) {
+    return fit_optimizer_launch(segs, num_segs, table, grad, grad_mul, grad2, scale2, scale2_mul, exp_avg, exp_avg_sq, n,
+                                lr, weight_decay, beta1, beta2, eps, step_small, step_table, scale, div, A_out,
+                                latent_dim, feature_dim, temperature, diff_sampling, seed, rng_step, w_hat, dw,
+                                ent_params, ent_layers, ent_noise, ent_seed, ent_rng_step, bits, grad_ent_params,
+                                ent_scratch, ent_scratch_bytes, ticket, nullptr, stream);
+}
+
+int shacira_fit_optimizer_step_best(const shacira_adam_seg_t* segs, int32_t num_segs, float* table, float* grad,
+                                    const float* grad_mul, const float* grad2, const float* scale2, float scale2_mul,
+                                    float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float weight_decay,
+                                    float beta1, float beta2, float eps, float* step_small, float* step_table,
+                                    const float* scale, const float* div, float* A_out, int32_t latent_dim,
+                                    int32_t feature_dim, const float* temperature, int32_t diff_sampling, uint64_t seed,
+                                    uint64_t* rng_step, float* w_hat, float* dw, const float* ent_params,
+                                    int32_t ent_layers, const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step,
+                                    double* bits, float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes,
+                                    uint32_t* ticket, const shacira_fit_snapshot_t* snap, shacira_stream_t stream) {
+    if (!snap) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_best: snapshot descriptor is NULL");
+    return fit_optimizer_launch(segs, num_segs, table, grad, grad_mul, grad2, scale2, scale2_mul, exp_avg, exp_avg_sq, n,
+                                lr, weight_decay, beta1, beta2, eps, step_small, step_table, scale, div, A_out,
+                                latent_dim, feature_dim, temperature, diff_sampling, seed, rng_step, w_hat, dw,
+                                ent_params, ent_layers, ent_noise, ent_seed, ent_rng_step, bits, grad_ent_params,
+                                ent_scratch, ent_scratch_bytes, ticket, snap, stream);
 }
 
 int shacira_multi_adam_step(const shacira_adam_seg_t* segs, int32_t num_segs, float beta1, float beta2, float eps,

@@ -27,6 +27,9 @@
 //
 // Shapes: 2D, latent_dim = feature_dim = 1, one affine decoder, 16 levels that all fit the tile's node box, rows in the
 // plan's sorted order (shacira_plan_set_sorted_io). Everything else keeps the three-kernel path.
+//
+// fit_render_kernel (end of file): the same tile walk, staging and lerp, forward only -- a model of this shape into pixels
+// and the integer SSE of its clamped PSNR (shacira_fit_render).
 #pragma once
 #include "mlp_tc_common.cuh"
 #include "tiled_kernels.cuh"
@@ -69,6 +72,35 @@ __device__ __forceinline__ void fit_locate(double t0, double t1, double resd, fl
     f0 = __fsub_rn(x, fx);
     f1 = __fsub_rn(y, fy);
     slot = offp + cx + cy * w0;
+}
+
+// This lane's entries of the first layer's A fragment: its 2 points x 4 levels lerped from the tile's staged nodes, with
+// the cell / weights of each kept for a backward scatter. Lane (g, t) owns points g, g+8 of its warp's 16 and the levels
+// lev[j] = 8 (j >> 1) + 2 t + (j & 1), i.e. fragment entry [j >> 1][2 hh + (j & 1)].
+__device__ __forceinline__ void fit_lerp(const double* resd_s, const float* hi_s, const TileGeom<2>& tg,
+                                         const int (&lev)[4], const double (&tu)[2][2], const float* s_nodes,
+                                         float Aval, float Sval, float (&X)[1][2][4], int (&slot)[2][4],
+                                         float (&f0)[2][4], float (&f1)[2][4]) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        const int l = lev[j];
+        const double resd = resd_s[l];
+        const float hi = hi_s[l];
+        const int offp = tg.offp[l], w0 = tg.w[l][0];
+#pragma unroll
+        for (int hh = 0; hh < 2; ++hh) {
+            fit_locate(tu[hh][0], tu[hh][1], resd, hi, offp, w0, slot[hh][j], f0[hh][j], f1[hh][j]);
+            const float g0 = __fsub_rn(1.0f, f0[hh][j]), g1 = __fsub_rn(1.0f, f1[hh][j]);
+            const int sb = slot[hh][j];
+            const float v0 = s_nodes[sb], v1 = s_nodes[sb + w0], v2 = s_nodes[sb + 1], v3 = s_nodes[sb + w0 + 1];
+            // corner order and contraction order of the tiled forward (stencil(), lerp_rows())
+            float z = __fmul_rn(v1, __fmul_rn(g0, f1[hh][j]));
+            z = __fmaf_rn(v0, __fmul_rn(g0, g1), z);
+            z = __fmaf_rn(v2, __fmul_rn(f0[hh][j], g1), z);
+            z = __fmaf_rn(v3, __fmul_rn(f0[hh][j], f1[hh][j]), z);
+            X[0][j >> 1][2 * hh + (j & 1)] = __fmaf_rn(z, Aval, Sval);
+        }
+    }
 }
 
 __global__ void __launch_bounds__(kTileThreads, SHACIRA_FIT_MIN_CTAS)
@@ -176,26 +208,7 @@ fit_tile_kernel(const PlanView pv, const float* __restrict__ latents, const __gr
             float X[1][2][4];
             int slot[2][4];
             float f0[2][4], f1[2][4];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const int l = lev[j];
-                const double resd = S.resd[l];
-                const float hi = S.hi[l];
-                const int offp = tg.offp[l], w0 = tg.w[l][0];
-#pragma unroll
-                for (int hh = 0; hh < 2; ++hh) {
-                    fit_locate(tu[hh][0], tu[hh][1], resd, hi, offp, w0, slot[hh][j], f0[hh][j], f1[hh][j]);
-                    const float g0 = __fsub_rn(1.0f, f0[hh][j]), g1 = __fsub_rn(1.0f, f1[hh][j]);
-                    const int sb = slot[hh][j];
-                    const float v0 = s_nodes[sb], v1 = s_nodes[sb + w0], v2 = s_nodes[sb + 1], v3 = s_nodes[sb + w0 + 1];
-                    // corner order and contraction order of the tiled forward (stencil(), lerp_rows())
-                    float z = __fmul_rn(v1, __fmul_rn(g0, f1[hh][j]));
-                    z = __fmaf_rn(v0, __fmul_rn(g0, g1), z);
-                    z = __fmaf_rn(v2, __fmul_rn(f0[hh][j], g1), z);
-                    z = __fmaf_rn(v3, __fmul_rn(f0[hh][j], f1[hh][j]), z);
-                    X[0][j >> 1][2 * hh + (j & 1)] = __fmaf_rn(z, Aval, Sval);
-                }
-            }
+            fit_lerp(S.resd, S.hi, tg, lev, tu, s_nodes, Aval, Sval, X, slot, f0, f1);
             // ---- MLP forward ------------------------------------------------------------------------------------------
             __syncwarp();   // the previous pass's weight-gradient reads of bufA are done
             tc_stage<1>(bufA, g, t, X);
@@ -448,6 +461,133 @@ fit_tile_kernel(const PlanView pv, const float* __restrict__ latents, const __gr
         const int dl = blockIdx.x % L;
         if (grad_A && S.gA != 0.0f) red_add(grad_A + dl, S.gA);
         if (grad_shift && S.gS != 0.0f) red_add(grad_shift + dl, S.gS);
+    }
+}
+
+// ---- forward only: grid -> MLP -> RGB (and the uint8 SSE against a target) ------------------------------------------------
+// fit_tile_kernel's tile walk, staging and lerp (fit_lerp) with rounding on -- the stored model is integers -- followed by
+// the 16 -> 16 -> 16 -> 3 forward on the tensor cores; nothing is staged for a backward. Rows follow the plan's convention
+// (original index, or tile order on a sorted-I/O plan). With `target`, every real output adds
+// (q(rgb) - q(target))^2 with q(v) = (uint8)(clamp(v, 0, 1) * 255) (torch's .to(torch.uint8) truncates): an integer sum,
+// exact in any order.
+struct RenderSmem {
+    uint4 wf[20][32];
+    double resd[16];
+    float hi[16];
+    float b1[16], b2[16], b3[4];
+};
+
+__device__ __forceinline__ int quantize_u8(float v) { return (int)__fmul_rn(fminf(fmaxf(v, 0.0f), 1.0f), 255.0f); }
+
+__global__ void __launch_bounds__(kTileThreads, SHACIRA_FIT_MIN_CTAS)
+fit_render_kernel(const PlanView pv, const float* __restrict__ latents, const __grid_constant__ LevelParams lp,
+                  const float* __restrict__ A, const float* __restrict__ shift, const float* __restrict__ W1,
+                  const float* __restrict__ b1, const float* __restrict__ W2, const float* __restrict__ b2,
+                  const float* __restrict__ W3, const float* __restrict__ b3, float* __restrict__ rgb,
+                  const float* __restrict__ target, unsigned long long* __restrict__ sse_u8, int cap) {
+    constexpr int OUT = 3;
+    extern __shared__ __align__(16) unsigned char s_raw[];
+    __shared__ TileGeom<2> tg;
+    RenderSmem& S = *reinterpret_cast<RenderSmem*>(s_raw);
+    float* s_nodes = reinterpret_cast<float*>(s_raw + sizeof(RenderSmem));   // [cap] rounded latents of the tile's nodes
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
+
+    tc_build_fragments(S.wf, W1, W2, W3, tid, kTileThreads);
+    if (tid < 16) {
+        S.b1[tid] = b1[tid];
+        S.b2[tid] = b2[tid];
+        S.resd[tid] = lp.resd[tid];
+        S.hi[tid] = lp.hi[tid];
+    }
+    if (tid < 4) S.b3[tid] = tid < OUT ? b3[tid] : 0.0f;
+    __syncthreads();
+    const float Aval = __ldg(A), Sval = shift ? __ldg(shift) : 0.0f;
+    int lev[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) lev[j] = 8 * (j >> 1) + 2 * t + (j & 1);
+    unsigned long long my_sse = 0ull;
+
+    for (int tile = blockIdx.x; tile < pv.ntiles; tile += gridDim.x) {
+        const int beg = pv.tile_off[tile], end = pv.tile_off[tile + 1];
+        if (beg == end) continue;   // uniform over the CTA
+        const int ti[2] = {tile % pv.g, tile / pv.g};
+        const int2* tab = pv.node_tab + (size_t)tile * pv.node_stride;
+        int pre[kPre];
+        prefetch_rows(tab, pv.node_stride, pre);
+        __syncthreads();   // the previous tile's passes are done with tg / s_nodes
+        tile_geometry<2>(tg, lp, ti, pv.g, cap);
+        stage_nodes_prefetched<2, 1>(tg, tab, pre, latents, 1, s_nodes);
+        __syncthreads();
+        for (int p0 = beg; p0 < end; p0 += kFitPts) {
+            const int base = p0 + warp * 16;
+            double tu[2][2];
+#pragma unroll
+            for (int hh = 0; hh < 2; ++hh) {
+                // rows past the tile's end take the tile's last point (valid slots); their outputs are dropped below
+                const float2 c = __ldg(reinterpret_cast<const float2*>(pv.coords_sorted) + min(base + g + 8 * hh, end - 1));
+                tu[hh][0] = unit_coord(c.x);
+                tu[hh][1] = unit_coord(c.y);
+            }
+            float X[1][2][4];
+            int slot[2][4];
+            float f0[2][4], f1[2][4];
+            fit_lerp(S.resd, S.hi, tg, lev, tu, s_nodes, Aval, Sval, X, slot, f0, f1);
+            float h1[1][2][4], h2[1][2][4];
+#pragma unroll
+            for (int nt = 0; nt < 2; ++nt) {
+                const float2 bb = *reinterpret_cast<const float2*>(&S.b1[8 * nt + 2 * t]);
+                h1[0][nt][0] = h1[0][nt][2] = bb.x;
+                h1[0][nt][1] = h1[0][nt][3] = bb.y;
+            }
+            tc_layer<2, 2, 1>(S.wf, F_L1, lane, X, h1);
+#pragma unroll
+            for (int nt = 0; nt < 2; ++nt) {
+                const float2 bb = *reinterpret_cast<const float2*>(&S.b2[8 * nt + 2 * t]);
+#pragma unroll
+                for (int r = 0; r < 4; ++r) h1[0][nt][r] = fmaxf(h1[0][nt][r], 0.0f);
+                h2[0][nt][0] = h2[0][nt][2] = bb.x;
+                h2[0][nt][1] = h2[0][nt][3] = bb.y;
+            }
+            tc_layer<2, 2, 1>(S.wf, F_L2, lane, h1, h2);
+#pragma unroll
+            for (int nt = 0; nt < 2; ++nt)
+#pragma unroll
+                for (int r = 0; r < 4; ++r) h2[0][nt][r] = fmaxf(h2[0][nt][r], 0.0f);
+            float Y[4];
+            {
+                const float2 bb = *reinterpret_cast<const float2*>(&S.b3[(2 * t) & 3]);
+                Y[0] = Y[2] = (t < 2) ? bb.x : 0.0f;
+                Y[1] = Y[3] = (t < 2) ? bb.y : 0.0f;
+#pragma unroll
+                for (int ks = 0; ks < 2; ++ks) {
+                    const uint4 f = S.wf[F_L3 + ks][lane];
+                    uint32_t ahi[4], alo[4];
+                    tile_to_a(h2[0][ks], ahi, alo);
+                    mma3(Y, ahi, alo, f.x, f.y, f.z, f.w);
+                }
+            }
+            // Y[r]: point base + g + 8 (r >> 1), column 2 t + (r & 1); columns < 3 are real
+            if (t < 2) {
+#pragma unroll
+                for (int r = 0; r < 4; ++r) {
+                    const int col = 2 * t + (r & 1);
+                    const int row = base + g + 8 * (r >> 1);
+                    if (col < OUT && row < end) {
+                        const int64_t o = (int64_t)(pv.perm ? __ldg(pv.perm + row) : row) * OUT + col;
+                        if (rgb) rgb[o] = Y[r];
+                        if (target) {
+                            const int d = quantize_u8(Y[r]) - quantize_u8(__ldg(target + o));
+                            my_sse += (unsigned long long)(d * d);
+                        }
+                    }
+                }
+            }
+        }
+    }
+    if (target) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) my_sse += __shfl_xor_sync(0xffffffffu, my_sse, o);
+        if (lane == 0 && my_sse) atomicAdd(sse_u8, my_sse);
     }
 }
 

@@ -50,11 +50,22 @@ struct TableAdam {
 };
 constexpr int kOptEnt = 13;   // bits | {d softplus(h), d b, d tanh(a)} x 4 layers
 
+// kSnap: best-state selection (shacira_fit_snapshot_t). The parameters are in registers right before their update, and
+// the arrival ticket orders every CTA's read of best_loss before the last CTA's write of it; kSnap = false compiles to
+// the kernel without it.
+template <bool kSnap>
 __global__ void __launch_bounds__(256)
 fit_optimizer_kernel(const __grid_constant__ AdamSegs S, const __grid_constant__ TableAdam Tb, float beta1, float beta2,
                      float eps, float* __restrict__ step_small, float* __restrict__ step_table,
                      const float* __restrict__ scale, const float* __restrict__ div, float* __restrict__ A_out, int C, int F,
-                     unsigned* __restrict__ ticket) {
+                     unsigned* __restrict__ ticket, const __grid_constant__ shacira_fit_snapshot_t snap) {
+    // this step's loss, bit for bit what ImageFitStep.rgb_loss() returns, against the best so far (NaN is never taken)
+    bool take = false;
+    float loss_t = 0.0f;
+    if constexpr (kSnap) {
+        loss_t = (float)(*snap.sse / (double)snap.count);
+        take = loss_t < *snap.best_loss;
+    }
     if ((int)blockIdx.x < S.num) {
         const float t = *step_small + 1.0f;
         const float bc1 = 1.0f - powf(beta1, t), inv_sqrt_bc2 = rsqrtf(1.0f - powf(beta2, t));
@@ -63,6 +74,14 @@ fit_optimizer_kernel(const __grid_constant__ AdamSegs S, const __grid_constant__
         const float step_size = sg.lr / bc1;
         // density-model segments wait for the bit-rate reduction when it runs in this launch (last CTA, below)
         const bool deferred = Tb.ent_params && sg.grad >= Tb.g_prob && sg.grad < Tb.g_prob + 12;
+        float* keep = nullptr;
+        if constexpr (kSnap) {
+            if (take) keep = snap.seg_param[blockIdx.x];
+            if (take && sg.param == scale) {   // the A this step's forward used, and the div it was made with
+                for (int e = threadIdx.x; e < C * F; e += 256) snap.A[e] = A_out[e];
+                for (int e = threadIdx.x; e < C; e += 256) snap.div[e] = div[e];
+            }
+        }
         for (int i = threadIdx.x; i < (deferred ? 0 : sg.n); i += 256) {
             float g = 0.0f;
             for (int r = 0; r < sg.grad_rows; ++r) g += sg.grad[(size_t)r * sg.grad_row_stride + i];
@@ -71,6 +90,9 @@ fit_optimizer_kernel(const __grid_constant__ AdamSegs S, const __grid_constant__
             g *= gs;
             if (sg.grad_div) g /= sg.grad_div[i / sg.div_group];
             const float p = sg.param[i];
+            if constexpr (kSnap) {
+                if (keep) keep[i] = p;
+            }
             const float gk = fmaf(sg.weight_decay, p, g);
             const float mk = fmaf(beta1, sg.exp_avg[i], (1.0f - beta1) * gk);
             const float vk = fmaf(beta2, sg.exp_avg_sq[i], (1.0f - beta2) * gk * gk);
@@ -138,6 +160,12 @@ fit_optimizer_kernel(const __grid_constant__ AdamSegs S, const __grid_constant__
                 P[k] = Tb.p[i4 + k]; M[k] = Tb.m[i4 + k]; V[k] = Tb.v[i4 + k]; G[k] = Tb.g[i4 + k];
                 if (Tb.gmul) Q[k] = Tb.gmul[i4 + k];
                 if (Tb.g2) H[k] = Tb.g2[i4 + k];
+            }
+        }
+        if constexpr (kSnap) {
+            if (take) {   // the continuous latents theta_t (under SGA the forward saw their sample)
+                if (vec) *reinterpret_cast<float4*>(snap.table + i4) = *reinterpret_cast<const float4*>(P);
+                else for (int k = 0; k < cnt; ++k) snap.table[i4 + k] = P[k];
             }
         }
         float s2e = s2;
@@ -309,12 +337,19 @@ fit_optimizer_kernel(const __grid_constant__ AdamSegs S, const __grid_constant__
                 const float t = *step_small + 1.0f;
                 const float bc1 = 1.0f - powf(beta1, t), inv_sqrt_bc2 = rsqrtf(1.0f - powf(beta2, t));
                 const float gs = sg.grad_mul * (sg.grad_scale ? *sg.grad_scale : 1.0f);
+                float* keep = nullptr;
+                if constexpr (kSnap) {
+                    if (take) keep = snap.seg_param[threadIdx.x];
+                }
                 for (int i = 0; i < sg.n; ++i) {
                     float g = 0.0f;
                     for (int r = 0; r < sg.grad_rows; ++r) g += sg.grad[(size_t)r * sg.grad_row_stride + i];
                     g *= gs;
                     if (sg.grad_div) g /= sg.grad_div[i / sg.div_group];
                     const float p = sg.param[i];
+                    if constexpr (kSnap) {
+                        if (keep) keep[i] = p;
+                    }
                     const float gk = fmaf(sg.weight_decay, p, g);
                     const float mk = fmaf(beta1, sg.exp_avg[i], (1.0f - beta1) * gk);
                     const float vk = fmaf(beta2, sg.exp_avg_sq[i], (1.0f - beta2) * gk * gk);
@@ -327,6 +362,12 @@ fit_optimizer_kernel(const __grid_constant__ AdamSegs S, const __grid_constant__
         __syncthreads();
     }
     if (threadIdx.x == 0) {
+        if constexpr (kSnap) {
+            if (take) {
+                *snap.best_loss = loss_t;
+                *snap.best_step = (int64_t)*step_small;
+            }
+        }
         *step_small += 1.0f;
         *step_table += 1.0f;
         if (Tb.w_hat && Tb.rng_step) *Tb.rng_step += 1ull;

@@ -567,4 +567,41 @@ int shacira_fit_tile_step(const shacira_plan_t* plan, const float* latents, cons
     return SHACIRA_OK;
 }
 
+int shacira_fit_render(const shacira_plan_t* plan, const float* latents, const int32_t* first_idx,
+                       const int32_t* resolutions, int32_t num_lods, int32_t codebook_bitwidth, const float* A,
+                       const float* shift, const float* W1, const float* b1, const float* W2, const float* b2,
+                       const float* W3, const float* b3, float* rgb, const float* target, uint64_t* sse_u8,
+                       shacira_stream_t stream) {
+    if (num_lods != 16) return fail(SHACIRA_ERR_UNSUPPORTED, "fit_render: 16 levels (got %d)", num_lods);
+    LevelParams lp;
+    int rc = build_levels(2, first_idx, resolutions, num_lods, codebook_bitwidth, lp);
+    if (rc) return rc;
+    if (!latents || !A || !W1 || !b1 || !W2 || !b2 || !W3 || !b3)
+        return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_render: NULL argument");
+    if (!rgb && !target) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_render: neither rgb nor target: nothing to compute");
+    if (target && !sse_u8) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_render: target needs sse_u8");
+    if (!plan) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "plan is NULL");
+    if (plan->dim != 2) return fail(SHACIRA_ERR_UNSUPPORTED, "fit_render: needs a 2D plan");
+    shacira_plan* p = const_cast<shacira_plan*>(plan);
+    // every level must live in the tile's node box (one float slot per node, no accumulators)
+    long long all = 0;
+    for (int l = 0; l < lp.num_lods; ++l) { const long long w = lp.res[l] / p->g + 3; all += w * w; }
+    const int cap_max = smem_budget() / 4;
+    if (all > cap_max) return fail(SHACIRA_ERR_UNSUPPORTED, "fit_render: %lld nodes per tile exceed the shared-memory box", all);
+    const int cap = node_capacity(p, lp, cap_max);
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((rc = ensure_node_table(p, lp, s))) return rc;
+    const size_t smem = sizeof(RenderSmem) + sizeof(float) * (size_t)cap;
+    static unsigned long long configured = 0ull;
+    if (needs_config(configured))
+        CUDA_OK(cudaFuncSetAttribute(fit_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+    if (target) CUDA_OK(cudaMemsetAsync(sse_u8, 0, sizeof(uint64_t), s));
+    int blocks = sm_count() * SHACIRA_FIT_MIN_CTAS;
+    if (blocks > p->ntiles) blocks = p->ntiles;
+    fit_render_kernel<<<blocks, kTileThreads, smem, s>>>(view_of(p), latents, lp, A, shift, W1, b1, W2, b2, W3, b3, rgb,
+                                                         target, (unsigned long long*)sse_u8, cap);
+    LAUNCHED();
+    return SHACIRA_OK;
+}
+
 }  // extern "C"

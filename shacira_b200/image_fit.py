@@ -26,8 +26,14 @@ the bit-rate noise is drawn in the kernel. The whole step is CUDA-graph capturab
 The module parameters stay the single source of truth: the kernels read and update the storage of
 `grid.codebook`, `grid.latent_dec.layers[0].{scale,shift}`, `grid.prob_model.f*.{h,b,a}` and the MLP in place, so
 `grid.interpolate`, `grid.size()`, `state_dict()` etc. see the trained values at any time.
+
+Model selection and evaluation stay on the device as well (image_trainer.py:173-178,305-310,471-502): with
+track_best=True the optimizer launch keeps the parameters of the lowest rgb_loss seen so far (`best_loss`, `best_step`,
+`restore_best`), and `render` / `render_image` turn a model of the fused kernel's shape into pixels and its clamped
+PSNR in one forward-only kernel (shacira_fit_render).
 """
 import ctypes
+import math
 import os
 
 import torch
@@ -38,13 +44,15 @@ from . import _lib, grid_ops
 class ImageFitStep:
     def __init__(self, grid, mlp, coords, target, lr=1e-3, grid_lr=2e-2, ldec_lr=1e-2, prob_lr=1e-4,
                  weight_decay=0.0, weight_decay_decoder=1e-2, betas=(0.9, 0.999), eps=1e-8, device_noise=False,
-                 noise_seed=0):
+                 noise_seed=0, track_best=False):
         """`grid`: shacira_b200.grids.LatentGrid (2D, single affine decoder; SGA sampling or STE rounding as the decoder's
         `use_sga` says -- see set_sga / set_temperature); `mlp`:
         nn.Sequential(Linear(L*F,16), ReLU, Linear(16,16), ReLU, Linear(16,3)); coords [N,2], target [N,3].
         Learning rates / weight decays: the reference's parameter groups (base_trainer.py:219-239; kodak.yaml:61-70).
         device_noise=True draws the bit-rate noise inside the kernel (fresh on every step, also under graph replay:
-        `draw_noise` is then unnecessary); False reads `self.noise`, which `draw_noise` fills (parity runs)."""
+        `draw_noise` is then unnecessary); False reads `self.noise`, which `draw_noise` fills (parity runs).
+        track_best=True keeps the state of the lowest rgb_loss inside the optimizer launch (see best_loss / restore_best);
+        it needs the one-launch optimizer (not SHACIRA_FIT_OPT_FUSED=0)."""
         dec = grid.latent_dec
         amap = dec.affine_map() if hasattr(dec, "affine_map") else None
         if amap is None or amap[0].shape[0] != 1 or "dft" in dec.layers[0].ldecode_matrix:
@@ -76,7 +84,8 @@ class ImageFitStep:
         # do not care about the order of the points, so grid and MLP exchange rows in the plan's tile order (targets
         # permuted once here) and the grid kernels lose their perm -> row dependent loads.
         self.plan = _lib.Plan(self.coords).set_sorted_io(True)
-        self.target = self.target[self.plan.perm_tensor()].contiguous()
+        self.perm = self.plan.perm_tensor()
+        self.target = self.target[self.perm].contiguous()
         f32 = dict(dtype=torch.float32, device=dev)
         # density-model parameters live in ONE [4, 3, C] buffer (the kernel's layout); the module's h / b / a become
         # views of it, so nothing is packed per step
@@ -98,6 +107,9 @@ class ImageFitStep:
         # one tile-resident kernel for grid forward + MLP / MSE + grid backward where its shapes apply (SHACIRA_FIT_FUSED=0:
         # the three-kernel path, kept for every other shape and as the parity reference of the fused kernel)
         self.opt_fused = os.environ.get("SHACIRA_FIT_OPT_FUSED", "1") != "0"   # one optimizer launch (incl. next SGA sample)
+        if track_best and not self.opt_fused:
+            raise _lib.ShaciraError(_lib.ERR_UNSUPPORTED, "ImageFitStep: track_best needs the one-launch optimizer "
+                                                          "(SHACIRA_FIT_OPT_FUSED=0 is set)")
         self._what_valid = False
         # the bit-rate loss evaluated inside the optimizer launch's table pass (latent_dim 1): no bit-rate launch, no
         # forked stream, the latents' bit-rate gradient never goes through memory
@@ -137,6 +149,7 @@ class ImageFitStep:
         self.step_small = torch.zeros((), **f32)
         self.adam_ticket = torch.zeros((), dtype=torch.int32, device=dev)   # arrival counter of the per-tensor CTAs
         self._keep = []
+        self._seg_params = []   # the tensor each Adam segment updates, in segment order (best-state snapshot)
         # the bit-rate kernel depends on nothing but the table: it runs on a forked stream beside the grid / MLP
         # kernels (it is latency bound: 17 us alone) and joins before the optimizer kernels
         self.side = torch.cuda.Stream(device=dev)
@@ -154,6 +167,7 @@ class ImageFitStep:
             s.n, s.grad_rows, s.grad_row_stride, s.div_group = n, rows, stride, group
             s.lr, s.weight_decay, s.grad_mul, s.zero_grad = lr, wd, mul, 1.0 if zero else 0.0
             segs.append(s)
+            self._seg_params.append(param)
 
         packed = self.mlp_out[2:2 + n_par]
         off = 0
@@ -191,6 +205,23 @@ class ImageFitStep:
         self.nseg = len(segs)
         self.layer = layer
         self.refresh_A()
+        self.track_best = bool(track_best)
+        if self.track_best:
+            # best-state snapshot, written by the optimizer launch on improving steps (shacira_fit_snapshot_t)
+            self.best_loss_t = torch.full((), float("inf"), **f32)
+            self.best_step_t = torch.full((), -1, dtype=torch.int64, device=dev)
+            self.best_table = torch.empty_like(grid.codebook.data)
+            self.best_segs = [torch.empty_like(p) for p in self._seg_params]
+            self.best_div = torch.empty_like(dec.div.data)
+            self.best_A = torch.empty_like(self.A)
+            snap = _lib.FitSnapshot()
+            snap.sse, snap.count = self.mlp_out.data_ptr(), self.n * self.OUT
+            snap.best_loss, snap.best_step = self.best_loss_t.data_ptr(), self.best_step_t.data_ptr()
+            snap.table, snap.div, snap.A = self.best_table.data_ptr(), self.best_div.data_ptr(), self.best_A.data_ptr()
+            for i, b in enumerate(self.best_segs):
+                snap.seg_param[i] = b.data_ptr()
+            self.snap = snap
+        self.sse_u8 = torch.zeros((), dtype=torch.int64, device=dev)
 
     # ---- host-side schedule hooks ------------------------------------------------------------
     def refresh_A(self):
@@ -302,32 +333,42 @@ class ImageFitStep:
                                                      P(self.g_prob), P(self.ent_scratch), self.ent_scratch.numel(),
                                                      _lib._stream()))
                 cur.wait_stream(self.side)
-            if self.opt_fused:
-                # ONE optimizer launch: small tensors + table Adam + the next step's SGA sample (csrc/optimizer_kernels.cuh)
-                chk(lib.shacira_fit_optimizer_step(ctypes.cast(self.segs, ctypes.c_void_p), self.nseg, P(lat), P(self.g_grid),
-                                                   P(gmul), None if ent_folded else P(self.g_ent), P(self.lam),
-                                                   1.0 / self.T, P(self.m_table),
-                                                   P(self.v_table), self.T * self.C, self.grid_lr, self.weight_decay,
-                                                   self.betas[0], self.betas[1], self.eps, P(self.step_small),
-                                                   P(self.step_table), P(self.layer.scale.data), P(dec.div.data), P(self.A),
-                                                   self.C, self.F, P(self.temperature), 1 if self.diff_sampling else 0,
-                                                   self.noise_seed + 0x5A17, P(self.sga_rng_step),
-                                                   P(self.w_hat) if prefetch else None, P(self.dw) if prefetch else None,
-                                                   P(self.prob) if ent_folded else None, self.num_prob_layers,
-                                                   None if self.device_noise else P(self.noise), self.noise_seed,
-                                                   P(self.rng_step), P(self.bits), P(self.g_prob), P(self.ent_scratch),
-                                                   self.ent_scratch.numel(), P(self.adam_ticket), st))
-                self._what_valid = prefetch
+            self._optimize(prefetch, gmul, ent_folded, st)
+
+    def _optimize(self, prefetch, gmul, ent_folded, st):
+        """The optimizer side of the step (one launch unless SHACIRA_FIT_OPT_FUSED=0)."""
+        lib, P, chk = _lib.load(), _lib._ptr, _lib._check
+        dec, lat = self.grid.latent_dec, self.grid.codebook.data
+        if self.opt_fused:
+            # ONE optimizer launch: small tensors + table Adam + the next step's SGA sample (csrc/optimizer_kernels.cuh)
+            args = [ctypes.cast(self.segs, ctypes.c_void_p), self.nseg, P(lat), P(self.g_grid),
+                    P(gmul), None if ent_folded else P(self.g_ent), P(self.lam),
+                    1.0 / self.T, P(self.m_table),
+                    P(self.v_table), self.T * self.C, self.grid_lr, self.weight_decay,
+                    self.betas[0], self.betas[1], self.eps, P(self.step_small),
+                    P(self.step_table), P(self.layer.scale.data), P(dec.div.data), P(self.A),
+                    self.C, self.F, P(self.temperature), 1 if self.diff_sampling else 0,
+                    self.noise_seed + 0x5A17, P(self.sga_rng_step),
+                    P(self.w_hat) if prefetch else None, P(self.dw) if prefetch else None,
+                    P(self.prob) if ent_folded else None, self.num_prob_layers,
+                    None if self.device_noise else P(self.noise), self.noise_seed,
+                    P(self.rng_step), P(self.bits), P(self.g_prob), P(self.ent_scratch),
+                    self.ent_scratch.numel(), P(self.adam_ticket)]
+            if self.track_best:   # the same launch, snapshotting the parameters of an improving step
+                chk(lib.shacira_fit_optimizer_step_best(*args, ctypes.byref(self.snap), st))
             else:
-                chk(lib.shacira_adam_step_sum_mul(P(lat), P(self.g_grid), P(gmul), P(self.g_ent), P(self.lam), 1.0 / self.T,
-                                                  P(self.m_table), P(self.v_table), self.T * self.C, self.grid_lr,
-                                                  self.betas[0], self.betas[1], self.eps, self.weight_decay,
-                                                  P(self.step_table), 0, 1, st))
-                chk(lib.shacira_multi_adam_step(ctypes.cast(self.segs, ctypes.c_void_p), self.nseg, self.betas[0],
-                                                self.betas[1], self.eps, P(self.step_small), P(self.step_table),
-                                                P(self.layer.scale.data), P(dec.div.data), P(self.A), self.C, self.F,
-                                                P(self.adam_ticket), st))
-                self._what_valid = False
+                chk(lib.shacira_fit_optimizer_step(*args, st))
+            self._what_valid = prefetch
+        else:
+            chk(lib.shacira_adam_step_sum_mul(P(lat), P(self.g_grid), P(gmul), P(self.g_ent), P(self.lam), 1.0 / self.T,
+                                              P(self.m_table), P(self.v_table), self.T * self.C, self.grid_lr,
+                                              self.betas[0], self.betas[1], self.eps, self.weight_decay,
+                                              P(self.step_table), 0, 1, st))
+            chk(lib.shacira_multi_adam_step(ctypes.cast(self.segs, ctypes.c_void_p), self.nseg, self.betas[0],
+                                            self.betas[1], self.eps, P(self.step_small), P(self.step_table),
+                                            P(self.layer.scale.data), P(dec.div.data), P(self.A), self.C, self.F,
+                                            P(self.adam_ticket), st))
+            self._what_valid = False
 
     # ---- results of the last step (device tensors; reading them synchronises) -------------------
     def rgb_loss(self):
@@ -336,7 +377,105 @@ class ImageFitStep:
     def total_bits(self):
         return self.bits[0].to(torch.float32)
 
+    # ---- best state (track_best=True) --------------------------------------------------------------
+    def _need_best(self):
+        if not self.track_best:
+            raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "ImageFitStep: constructed without track_best=True")
+
+    def best_loss(self):
+        """Lowest rgb_loss() over the steps so far (+inf before the first step): float32 device scalar."""
+        self._need_best()
+        return self.best_loss_t.clone()
+
+    def best_step(self):
+        """0-based index of the step (call of step()) that produced best_loss(); -1 before the first step."""
+        self._need_best()
+        return self.best_step_t.clone()
+
+    def restore_best(self):
+        """Copy the best state into the module parameters in place: latent table, MLP, latent decoder, density model,
+        div and A, as they were when that step's forward ran (the reference reloads its best model, not the optimizer
+        state: the Adam moments stay as they are). Reads best_step() on the host."""
+        self._need_best()
+        if int(self.best_step_t) < 0:
+            raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "ImageFitStep.restore_best: no step has been taken")
+        with torch.no_grad():
+            self.grid.codebook.data.copy_(self.best_table)
+            for p, b in zip(self._seg_params, self.best_segs):
+                p.copy_(b)
+            self.grid.latent_dec.div.data.copy_(self.best_div)
+            self.A.copy_(self.best_A)
+        self._what_valid = False   # the prefetched SGA sample belongs to the replaced latents
+
+    # ---- evaluation ------------------------------------------------------------------------------------
+    def render(self, target=True):
+        """(rgb [N, 3] in the caller's coordinate order, clamped PSNR as a float64 device scalar or None) of the current
+        parameters, rounding the latents (the stored model is integers): one kernel over the step's own plan."""
+        rgb = torch.empty((self.n, self.OUT), dtype=torch.float32, device=self.dev)
+        with torch.cuda.device(self.dev):
+            _render(self.plan, self.grid.codebook.data, self.fi, self.rs, self.L, self.bw, self.A,
+                    self.layer.shift.data if self.has_shift else None, self.lin, rgb,
+                    self.target if target else None, self.sse_u8)
+            out = torch.empty_like(rgb)
+            out[self.perm] = rgb       # tile order -> original order
+        return out, (_psnr(self.sse_u8, self.n * self.OUT) if target else None)
+
     def close(self):
         if self.plan is not None:
             self.plan.close()
             self.plan = None
+
+
+def _render(plan, latents, fi, rs, L, bw, A, shift, lin, rgb, target, sse):
+    P = _lib._ptr
+    _lib._check(_lib.load().shacira_fit_render(plan.handle, P(latents), fi, rs, L, bw, P(A), P(shift),
+                                               P(lin[0].weight.data), P(lin[0].bias.data), P(lin[1].weight.data),
+                                               P(lin[1].bias.data), P(lin[2].weight.data), P(lin[2].bias.data), P(rgb),
+                                               P(target), P(sse) if target is not None else None, _lib._stream()))
+
+
+def _psnr(sse, count):
+    """clamped_psnr of wisp/ops/image/metrics.py:39-57 from the integer uint8 SSE (device float64 scalar)."""
+    mse = torch.clamp(sse.to(torch.float64) / count, min=1e-12)
+    return 20.0 * math.log10(255.0) - 10.0 * torch.log10(mse)
+
+
+def render_image(grid, mlp, coords, target=None):
+    """mlp(grid.interpolate(coords)) for a model of the fused fit kernel's shape -- 2D LatentGrid with 16 levels,
+    latent_dim = feature_dim = 1, one affine 'sq' latent decoder, MLP 16 -> 16 -> 16 -> 3 -- in one forward-only kernel
+    with the latents rounded: a trained or a decoded codec model, on any coordinate set (e.g. a 2x upsampled pixel
+    grid). Returns (rgb [N, 3] in the order of `coords`, clamped PSNR against `target` [N, 3] as a float64 device
+    scalar, or None without a target). Other shapes raise ShaciraError (use mlp(grid.interpolate(coords)))."""
+    dec = grid.latent_dec
+    amap = dec.affine_map() if hasattr(dec, "affine_map") else None
+    lin = [mlp[0], mlp[2], mlp[4]] if len(mlp) == 5 else None
+    if (amap is None or amap[0].shape[0] != 1 or "dft" in getattr(dec.layers[0], "ldecode_matrix", "") or
+            grid.resolution_dim != 2 or grid.num_lods != 16 or tuple(grid.codebook.shape[1:]) != (1,) or
+            tuple(amap[0].shape) != (1, 1, 1) or lin is None or
+            [(l.in_features, l.out_features) for l in lin] != [(16, 16), (16, 16), (16, 3)]):
+        raise _lib.ShaciraError(_lib.ERR_UNSUPPORTED, "render_image: needs the fused fit kernel's model shape")
+    coords = _lib._f32c(coords, "coords")
+    n = coords.shape[0]
+    if coords.dim() != 2 or coords.shape[1] != 2:
+        raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "render_image: coords must be [N, 2]")
+    if target is not None:
+        target = _lib._f32c(target, "target")
+        if tuple(target.shape) != (n, 3):
+            raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "render_image: target must be [N, 3]")
+    # the cached plan of these coordinates; small sets get a plan of their own with small tiles, so that every level's
+    # node box fits a tile's shared memory
+    plan = grid_ops.plan_for(coords) if coords.shape[0] >= grid_ops.PLAN_MIN_POINTS else None
+    if plan is None:
+        plan = _lib.Plan(coords, tile_points=32)
+    fi, _ = _lib._i32_array(grid._first_idx())
+    rs, L = _lib._i32_array(grid.resolutions)
+    A, shift = amap
+    with torch.no_grad():
+        A = A.detach().contiguous()
+        shift = shift.detach().contiguous() if shift is not None else None
+    rgb = torch.empty((n, 3), dtype=torch.float32, device=coords.device)
+    sse = torch.zeros((), dtype=torch.int64, device=coords.device) if target is not None else None
+    with torch.cuda.device(coords.device):
+        _render(plan, _lib._f32c(grid.codebook.data, "codebook"), fi, rs, L, int(grid.codebook_bitwidth), A, shift, lin,
+                rgb, target, sse)
+    return rgb, (_psnr(sse, n * 3) if target is not None else None)
