@@ -13,10 +13,22 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from shacira_b200 import _lib  # noqa: E402
 from shacira_b200.grids import geometric_resolutions  # noqa: E402
-from probe3d import timed  # noqa: E402
 
 dev = torch.device("cuda", 0)
 lib = _lib.load()
+
+
+def timed(fn, iters=12, warm=3):
+    for i in range(warm):
+        fn(i)
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for i in range(iters):
+        fn(i)
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / iters * 1e3
 
 
 def layout(res, bw, dim):

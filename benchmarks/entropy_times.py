@@ -1,5 +1,5 @@
 """Device time of the bit-rate kernel: training mode (noise buffer / in-kernel noise) and validation mode, at the image
-table (374 612 rows) and the NeRF table (6 098 925 rows). SHACIRA_ENT_HIST=0 disables the validation-mode histogram."""
+table (374 612 rows) and the NeRF table (6 098 925 rows)."""
 import json
 import os
 import sys
@@ -9,10 +9,9 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from shacira_b200 import _lib  # noqa: E402
-from probe3d import timed  # noqa: E402
 
 dev = torch.device("cuda", 0)
-out = {"hist": os.environ.get("SHACIRA_ENT_HIST", "1")}
+out = {}
 for name, T, L in (("image", 374612, 16), ("nerf", 6098925, 16), ("nerf_total_only", 6098925, 0)):
     torch.manual_seed(0)
     w = torch.randn(T, 1, device=dev) * 6

@@ -1,6 +1,6 @@
 """Device time of the 3D kernels at the NeRF shape (BASELINE cfg4: 2^19 samples, 16 levels 16->2048, 2^19-row
 tables, C=1 -> F=4) and the plain HashGrid shape (F=2): CUDA events around 20 launches after 5 warm-ups, four rotating
-input sets (4 x 160 MB > L2). SHACIRA_COARSE_MAX_SLABS=0 turns the shared-memory coarse-level backward off (A/B).
+input sets (4 x 160 MB > L2).
 
     python benchmarks/kernel_times_3d.py [--n 524288] [--bw 19]
 """
@@ -50,7 +50,7 @@ def main():
     rs, _ = _lib._i32_array(res)
     P = _lib._ptr
     torch.manual_seed(0)
-    out = {"n": S, "bw": BW, "rows": T, "coarse_max_slabs": os.environ.get("SHACIRA_COARSE_MAX_SLABS", "default")}
+    out = {"n": S, "bw": BW, "rows": T}
     for name, C, F in (("latent_c1_f4", 1, 4), ("plain_f2", 2, 2)):
         sets = [dict(coords=torch.rand((S, 3), device=dev) * 2 - 1, g=torch.randn((S, L * F), device=dev)) for _ in range(4)]
         lat = (torch.rand((T, C), device=dev) - 0.5) * 16

@@ -1,6 +1,5 @@
 """A few launches of the 3D (NeRF-shape, cfg4) kernels for an ncu capture.
-    ncu --set full ... python benchmarks/ncu_3d.py [--sorted TILE_POINTS] [--what fwd|bwd|both]
-Environment: SHACIRA_3D_MERGE / SHACIRA_3D_RED / SHACIRA_3D_STAGED select the variant."""
+    ncu --set full ... python benchmarks/ncu_3d.py [--sorted TILE_POINTS] [--what fwd|bwd|both]"""
 import argparse
 import os
 import sys

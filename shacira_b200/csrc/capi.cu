@@ -1,6 +1,5 @@
 // capi.cu -- the extern "C" surface declared in include/shacira_b200.h: argument validation,
 // level metadata, template dispatch and launches. No torch, no exceptions across the ABI.
-#include <cstdlib>
 
 #include "arith_coder.inl"
 #include "capi_internal.h"
@@ -82,23 +81,16 @@ inline int grid_for(int64_t n, int block) { return (int)((n + block - 1) / block
 template <int D, int F>
 int launch_plain_fwd(const float* coords, int64_t n, const float* table, const LevelParams& lp, float* feats,
                      cudaStream_t s) {
-    if (D == 3 && grid3d_merge_mode() >= 2 && grid3d_supported(F, F, table))   // lane pairs, identity decoder
+    if (D == 3 && grid3d_supported(F, F, table))   // lane pairs, identity decoder
         return launch_fwd3d(F, F, coords, nullptr, n, table, lp, nullptr, nullptr, 0, 0, feats, nullptr, s);
     hashgrid_fwd_kernel<D, F><<<grid_for(n, kBlock), kBlock, 0, s>>>(coords, n, table, lp, feats);
     LAUNCHED();
     return SHACIRA_OK;
 }
 // Coarse dense levels go through shared memory (coarse_kernels.cuh) when the batch is large enough for their
-// same-address global adds to serialise; SHACIRA_COARSE_MAX_SLABS=0 turns the path off (tuning / A-B runs).
-inline int coarse_max_slabs() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SHACIRA_COARSE_MAX_SLABS");
-        v = e ? atoi(e) : 1;  // measured at the NeRF shape: whole-level jobs pay, slabbed levels do not
-        if (v < 0) v = 0;
-    }
-    return v;
-}
+// same-address global adds to serialise. One slab per level: measured at the NeRF shape, whole-level jobs pay,
+// slabbed levels do not.
+constexpr int kCoarseMaxSlabs = 1;
 inline int join_side(cudaStream_t s) {
     SideStream* ss = nullptr;
     if (int rc = side_stream(&ss)) return rc;
@@ -111,10 +103,10 @@ int launch_coarse_bwd(const float* coords, int64_t n, const float* g, const Leve
                       uint32_t level_mask = 0xffffffffu) {
     mask = 0;
     pending_join = false;
-    if (n < 65536 || coarse_max_slabs() == 0) return SHACIRA_OK;
+    if (n < 65536) return SHACIRA_OK;
     CoarseJobs jobs;
     constexpr int NV = LATENT ? C : F;
-    const uint32_t m = plan_coarse_jobs(D, lp, NV, n, sm_count(), coarse_max_slabs(), jobs, level_mask);
+    const uint32_t m = plan_coarse_jobs(D, lp, NV, n, sm_count(), kCoarseMaxSlabs, jobs, level_mask);
     if (!m) return SHACIRA_OK;
     const size_t smem = coarse_smem_bytes(jobs, NV);
     static unsigned long long configured = 0ull;
@@ -124,14 +116,6 @@ int launch_coarse_bwd(const float* coords, int64_t n, const float* g, const Leve
     // The coarse kernel is bound by shared-memory CAS, the point-parallel kernel by L2 atomics: fork a side stream so
     // that both run at once (one coarse CTA per SM is placed first, the other kernel fills the rest of the SM).
     // Event fork/join composes with stream capture (the side stream joins the caller's capture).
-    static const bool fork = [] { const char* e = getenv("SHACIRA_COARSE_FORK"); return !e || atoi(e) != 0; }();
-    if (!fork) {  // A/B runs: same stream, the two kernels serialise
-        coarse_bwd_kernel<D, C, F, LATENT><<<coarse_total_ctas(jobs), kCoarseThreads, smem, s>>>(
-            coords, n, g, lp, jobs, A, per_level, gt);
-        LAUNCHED();
-        mask = m;
-        return SHACIRA_OK;
-    }
     SideStream* ssp = nullptr;
     if (int rc = side_stream(&ssp)) return rc;
     SideStream& ss = *ssp;
@@ -152,8 +136,8 @@ int launch_plain_bwd(const float* coords, int64_t n, const float* g, const Level
     bool join = false;
     int rc = launch_coarse_bwd<D, F, F, false>(coords, n, g, lp, nullptr, 0, gt, s, skip, join);
     if (rc) return rc;
-    if (D == 3 && grid3d_red_mode() >= 8 && grid3d_supported(F, F, gt)) {   // lane pairs, identity decoder
-        rc = launch_bwd3d(F, F, coords, nullptr, n, g, nullptr, lp, nullptr, 0, skip, 0xffffffffu, 8, gt, nullptr, nullptr, s);
+    if (D == 3 && grid3d_supported(F, F, gt)) {   // lane pairs, identity decoder
+        rc = launch_bwd3d(F, F, coords, nullptr, n, g, nullptr, lp, nullptr, 0, skip, 0xffffffffu, gt, nullptr, nullptr, s);
         if (rc) return rc;
         return join ? join_side(s) : SHACIRA_OK;
     }
@@ -165,7 +149,7 @@ template <int D, int C, int F>
 int launch_latent_fwd(const float* coords, int64_t n, const float* lat, const LevelParams& lp, const float* A,
                       const float* shift, int per_level, int round_flag, float* feats, float* zsave,
                       cudaStream_t s) {
-    if (D == 3 && grid3d_merge_mode() > 0 && grid3d_supported(C, F, lat))   // merged x-pair loads (grid3d_kernels.cuh)
+    if (D == 3 && grid3d_supported(C, F, lat))   // lane pairs (grid3d_kernels.cuh)
         return launch_fwd3d(C, F, coords, nullptr, n, lat, lp, A, shift, per_level, round_flag, feats, zsave, s);
     const int nA = per_level ? lp.num_lods : 1;
     const size_t smem = sizeof(float) * (size_t)(nA * C * F + nA * F);
@@ -184,9 +168,8 @@ int launch_latent_bwd(const float* coords, int64_t n, const float* g, const floa
     bool join = false;
     int rc = launch_coarse_bwd<D, C, F, true>(coords, n, g, lp, A, per_level, gl, s, skip, join, level_mask);
     if (rc) return rc;
-    if (D == 3 && grid3d_red_mode() >= 0 && grid3d_supported(C, F, gl)) {   // vector reds per x-pair (grid3d_kernels.cuh)
-        rc = launch_bwd3d(C, F, coords, nullptr, n, g, zsave, lp, A, per_level, skip, level_mask, grid3d_red_mode(), gl,
-                          gA, gS, s);
+    if (D == 3 && grid3d_supported(C, F, gl)) {   // lane pairs (grid3d_kernels.cuh)
+        rc = launch_bwd3d(C, F, coords, nullptr, n, g, zsave, lp, A, per_level, skip, level_mask, gl, gA, gS, s);
         if (rc) return rc;
         return join ? join_side(s) : SHACIRA_OK;
     }
@@ -216,53 +199,18 @@ int launch_latent_bwd(const float* coords, int64_t n, const float* g, const floa
 }  // namespace
 
 namespace {
-// IN = 16: weights as constant-bank operands (mlp16_mse_step_kernel). The six tensors are copied device-to-device
-// into the constant bank on the caller's stream (one copy when they are packed back to back, as ImageFitStep keeps
-// them); the copies are stream ordered and capturable.
-int launch_mlp16(const float* x, const float* gt, int64_t n, const float* W1, const float* b1, const float* W2,
-                 const float* b2, const float* W3, const float* b3, float* gx, float* pred, void* out, cudaStream_t s) {
-    static unsigned long long configured = 0ull;
-    if (needs_config(configured))
-        CUDA_OK(cudaFuncSetAttribute(mlp16_mse_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)sizeof(Mlp16Smem)));
-    const float* src[6] = {W1, b1, W2, b2, W3, b3};
-    const size_t cnt[6] = {256, 16, 256, 16, 48, 3};
-    bool packed = true;
-    for (int k = 0; k + 1 < 6; ++k) packed &= (src[k] + cnt[k] == src[k + 1]);
-    if (packed) {
-        CUDA_OK(cudaMemcpyToSymbolAsync(shacira_c_mlp, W1, sizeof(float) * kMlpConstFloats, 0, cudaMemcpyDeviceToDevice, s));
-    } else {
-        size_t off = 0;
-        for (int k = 0; k < 6; ++k) {
-            CUDA_OK(cudaMemcpyToSymbolAsync(shacira_c_mlp, src[k], sizeof(float) * cnt[k], sizeof(float) * off,
-                                            cudaMemcpyDeviceToDevice, s));
-            off += cnt[k];
-        }
-    }
-    const size_t out_bytes = 8 + sizeof(float) * kMlpConstFloats;
-    CUDA_OK(cudaMemsetAsync(out, 0, out_bytes, s));
-    int64_t warps = (n + 31) / 32;
-    int64_t blocks = (warps + kMlpWarps - 1) / kMlpWarps;
-    const int64_t cap = (int64_t)sm_count() * 2;  // persistent: 2 CTAs per SM fit the shared memory
-    if (blocks > cap) blocks = cap;
-    const float scale = (float)(2.0 / ((double)n * 3.0));
-    mlp16_mse_step_kernel<<<(int)blocks, kMlpThreads, sizeof(Mlp16Smem), s>>>(x, gt, n, scale, gx, pred, (double*)out,
-                                                                              (float*)((char*)out + 8));
-    LAUNCHED();
-    return SHACIRA_OK;
-}
-
-// IN = 16 on the tensor cores (mlp16_tc_step_kernel: mma.sync TF32 with 3xTF32 compensation)
-template <int MT, int WARPS, int MINB>
-int launch_mlp_tc_cfg(const float* x, const float* gt, int64_t n, const float* W1, const float* b1, const float* W2,
-                      const float* b2, const float* W3, const float* b3, float* gx, float* pred, void* out, float* absmax,
-                      cudaStream_t s) {
+// IN = 16 on the tensor cores (mlp16_tc_step_kernel: mma.sync TF32 with 3xTF32 compensation). Two m16 tiles per warp
+// iteration, 6 warps x 2 CTAs per SM: the configuration chosen by measurement (mlp_kernels.cuh).
+int launch_mlp_tc(const float* x, const float* gt, int64_t n, const float* W1, const float* b1, const float* W2,
+                  const float* b2, const float* W3, const float* b3, float* gx, float* pred, void* out, float* absmax,
+                  cudaStream_t s) {
+    constexpr int MT = 2, WARPS = 6, MINB = 2;
     using Smem = MlpTcSmem<MT, WARPS>;
     static unsigned long long configured = 0ull;
     if (needs_config(configured))
         CUDA_OK(cudaFuncSetAttribute(mlp16_tc_step_kernel<MT, WARPS, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)sizeof(Smem)));
-    const size_t out_bytes = 8 + sizeof(float) * kMlpConstFloats;
+    const size_t out_bytes = 8 + sizeof(float) * kMlp16Params;
     if (absmax && (char*)absmax == (char*)out + out_bytes) {   // caller keeps the bound behind `out`: one memset node
         CUDA_OK(cudaMemsetAsync(out, 0, out_bytes + sizeof(float) * 16, s));
     } else {
@@ -278,17 +226,6 @@ int launch_mlp_tc_cfg(const float* x, const float* gt, int64_t n, const float* W
         x, gt, n, W1, b1, W2, b2, W3, b3, scale, gx, pred, (double*)out, (float*)((char*)out + 8), (unsigned*)absmax);
     LAUNCHED();
     return SHACIRA_OK;
-}
-
-// IN = 16 on the tensor cores (mlp16_tc_step_kernel: mma.sync TF32 with 3xTF32 compensation)
-int launch_mlp_tc(const float* x, const float* gt, int64_t n, const float* W1, const float* b1, const float* W2,
-                  const float* b2, const float* W3, const float* b3, float* gx, float* pred, void* out, float* absmax,
-                  cudaStream_t s) {
-    // SHACIRA_MLP_MT: 2 = two m16 tiles per warp iteration, 6 warps x 2 CTAs per SM; 1 = one tile, 6 warps x 3 CTAs (11: 8 warps x 2 CTAs)
-    static const int mt = [] { const char* e = getenv("SHACIRA_MLP_MT"); return e ? atoi(e) : 2; }();
-    if (mt == 1) return launch_mlp_tc_cfg<1, 6, 3>(x, gt, n, W1, b1, W2, b2, W3, b3, gx, pred, out, absmax, s);
-    if (mt == 11) return launch_mlp_tc_cfg<1, 8, 2>(x, gt, n, W1, b1, W2, b2, W3, b3, gx, pred, out, absmax, s);
-    return launch_mlp_tc_cfg<2, 6, 2>(x, gt, n, W1, b1, W2, b2, W3, b3, gx, pred, out, absmax, s);
 }
 
 template <int IN>
@@ -499,8 +436,7 @@ static int entropy_bits_impl(const float* latents, const float* noise, int64_t t
     lb.first[num_lods] = (int32_t)table_rows;
     const int sms = sm_count();
     int64_t blocks = (total + kEntBlock - 1) / kEntBlock;
-    static const int per_sm = [] { const char* e = getenv("SHACIRA_ENT_BLOCKS_PER_SM"); int v = e ? atoi(e) : 0; return v > 0 ? v : 4; }();
-    const int64_t cap = (int64_t)sms * per_sm;  // per-block prologue/epilogue (~500 instructions) vs parallelism: tuned on B200
+    const int64_t cap = (int64_t)sms * 4;  // per-block prologue/epilogue (~500 instructions) vs parallelism: tuned on B200
     if (blocks > cap) blocks = cap;
     // scratch: [0, 256) arrival ticket, then the block partials. The ticket sits at a FIXED offset: one scratch serves
     // launches of any table size (a ticket behind the partials would be overwritten by a larger launch's rows). The
@@ -517,11 +453,10 @@ static int entropy_bits_impl(const float* latents, const float* noise, int64_t t
     }
     unsigned* ticket = (unsigned*)buf;
     // validation mode (x = round(w)): per-integer table in shared memory instead of per-element CDF chains
-    static const bool lut_on = [] { const char* e = getenv("SHACIRA_ENT_LUT"); return !e || atoi(e) != 0; }();
     const bool val_mode = !noise && !rng_step;
     // (pays from ~1 M entries: every CTA builds the table first -- measured 22.9 vs 17.1 us at the image table's 375 k,
     // 51.6 vs 85.7 us at the NeRF table's 6.1 M with per-level sums)
-    if (val_mode && lut_on && latent_dim <= 4 && total >= (1 << 20)) {
+    if (val_mode && latent_dim <= 4 && total >= (1 << 20)) {
         const size_t lut_bytes = sizeof(float) * (size_t)latent_dim * kLutK * kLutN;
         if (lut_bytes > 48 * 1024) {
             static unsigned long long configured = 0ull;
@@ -828,19 +763,8 @@ int shacira_mlp_mse_step_bounded(const float* features, const float* target, int
         return fail(SHACIRA_ERR_UNSUPPORTED, "mlp_mse_step: hidden %d / out %d (compiled: 16 / 3)", hidden_dim, out_dim);
     cudaStream_t s = (cudaStream_t)stream;
     switch (in_dim) {
-        case 16: {
-            // SHACIRA_MLP_IMPL = tc (default) | const (FFMA, weights in the constant bank) | smem (FFMA, shared memory)
-            static const int impl = [] {
-                const char* e = getenv("SHACIRA_MLP_IMPL");
-                return !e ? 0 : (!strcmp(e, "const") ? 1 : (!strcmp(e, "smem") ? 2 : 0));
-            }();
-            if (grad_feature_absmax && impl != 0)
-                return fail(SHACIRA_ERR_UNSUPPORTED, "mlp_mse_step_bounded: only the tensor-core kernel reduces the bound");
-            if (impl == 2) return launch_mlp<16>(features, target, n, W1, b1, W2, b2, W3, b3, grad_features, pred, out, s);
-            if (impl == 1) return launch_mlp16(features, target, n, W1, b1, W2, b2, W3, b3, grad_features, pred, out, s);
-            return launch_mlp_tc(features, target, n, W1, b1, W2, b2, W3, b3, grad_features, pred, out,
-                                 grad_feature_absmax, s);
-        }
+        case 16: return launch_mlp_tc(features, target, n, W1, b1, W2, b2, W3, b3, grad_features, pred, out,
+                                      grad_feature_absmax, s);
         case 24: if (grad_feature_absmax) return fail(SHACIRA_ERR_UNSUPPORTED, "mlp_mse_step_bounded: in_dim 16 only");
                  return launch_mlp<24>(features, target, n, W1, b1, W2, b2, W3, b3, grad_features, pred, out, s);
         case 32: if (grad_feature_absmax) return fail(SHACIRA_ERR_UNSUPPORTED, "mlp_mse_step_bounded: in_dim 16 only");

@@ -104,20 +104,16 @@ inline int side_stream(SideStream** out) {
     return SHACIRA_OK;
 }
 
-// 3D kernels with merged x-pair accesses (grid3d_kernels.cuh, launched from grid3d_capi.cu). `perm` != NULL: `coords`
-// is a plan's sorted copy and row i of feats / grad_output belongs to sample perm[i]; zsave rows follow `coords`.
-// *_supported: latent_dim 1 or 2 and 16-byte aligned tables (the merged accesses are aligned 16-byte vectors).
+// 3D lane-pair kernels (grid3d_kernels.cuh, launched from grid3d_capi.cu). `perm` != NULL: `coords` is a plan's
+// sorted copy and row i of feats / grad_output belongs to sample perm[i]; zsave rows follow `coords`.
+// *_supported: latent_dim 1 or 2 and 16-byte aligned tables.
 bool grid3d_supported(int latent_dim, int feature_dim, const void* table);
 int launch_fwd3d(int latent_dim, int feature_dim, const float* coords, const int32_t* perm, int64_t n,
                  const float* latents, const LevelParams& lp, const float* A, const float* shift, int per_level,
                  int round_flag, float* feats, float* zsave, cudaStream_t s);
-// red_w: 4 / 2 = vector reds on the aligned quad / pair, 0 = one red per corner
 int launch_bwd3d(int latent_dim, int feature_dim, const float* coords, const int32_t* perm, int64_t n,
                  const float* grad_out, const float* zsave, const LevelParams& lp, const float* A, int per_level,
-                 uint32_t skip_mask, uint32_t level_mask, int red_w, float* grad_latents, float* grad_A,
-                 float* grad_shift, cudaStream_t s, int ctas_per_sm = 4);
-// tuning knobs (environment, read per call: A/B runs flip them inside one process)
-int grid3d_merge_mode();   // SHACIRA_3D_MERGE: 1 (default) = merged forward loads, 0 = point-parallel kernel
-int grid3d_red_mode();     // SHACIRA_3D_RED:   4 (default) / 2 = vector reds, 0 = scalar, -1 = point-parallel kernel
+                 uint32_t skip_mask, uint32_t level_mask, float* grad_latents, float* grad_A, float* grad_shift,
+                 cudaStream_t s, int ctas_per_sm = 4);
 
 }  // namespace shacira

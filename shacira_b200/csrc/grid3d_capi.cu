@@ -1,20 +1,9 @@
-// grid3d_capi.cu -- launchers of the 3D kernels with merged x-pair accesses (grid3d_kernels.cuh); declared in
+// grid3d_capi.cu -- launchers of the 3D lane-pair kernels (grid3d_kernels.cuh); declared in
 // capi_internal.h and used by the unplanned (capi.cu) and planned (tiled_capi.cu) entry points.
-#include <cstdlib>
-
 #include "capi_internal.h"
 #include "grid3d_kernels.cuh"
 
 namespace shacira {
-
-int grid3d_merge_mode() {
-    const char* e = getenv("SHACIRA_3D_MERGE");
-    return e ? atoi(e) : 2;
-}
-int grid3d_red_mode() {
-    const char* e = getenv("SHACIRA_3D_RED");
-    return e ? atoi(e) : 8;
-}
 
 bool grid3d_supported(int latent_dim, int feature_dim, const void* table) {
     if (latent_dim != 1 && latent_dim != 2) return false;
@@ -37,50 +26,34 @@ template <int C, int F>
 int fwd3d(const float* coords, const int32_t* perm, int64_t n, const float* lat, const LevelParams& lp, const float* A,
           const float* shift, int per_level, int round_flag, float* feats, float* zsave, cudaStream_t s) {
     const int nA = per_level ? lp.num_lods : 1;
-    if (!A && (C != F || grid3d_merge_mode() < 2)) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "3D forward: A is NULL");
-    if (grid3d_merge_mode() >= 2) {   // lane pairs
-        const size_t smem = LpFwdLayout<C, F>::bytes(nA);
-        static unsigned long long configured = 0ull;
-        if (needs_config(configured))
-            CUDA_OK(cudaFuncSetAttribute(latent_fwd3d_lp_kernel<C, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-        latent_fwd3d_lp_kernel<C, F><<<grid_for(n, kLpChunk), kLpBlock, smem, s>>>(coords, perm, n, lat, lp, A, shift,
-                                                                                    per_level, round_flag, feats, zsave);
-        LAUNCHED();
-        return SHACIRA_OK;
-    }
-    const size_t smem = sizeof(float) * (size_t)(nA * C * F + nA * F);
-    latent_fwd3d_kernel<C, F><<<grid_for(n, kBlock), kBlock, smem, s>>>(coords, perm, n, lat, lp, A, shift, per_level,
-                                                                         round_flag, feats, zsave);
+    if (!A && C != F) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "3D forward: A is NULL");
+    const size_t smem = LpFwdLayout<C, F>::bytes(nA);
+    static unsigned long long configured = 0ull;
+    if (needs_config(configured))
+        CUDA_OK(cudaFuncSetAttribute(latent_fwd3d_lp_kernel<C, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+    latent_fwd3d_lp_kernel<C, F><<<grid_for(n, kLpChunk), kLpBlock, smem, s>>>(coords, perm, n, lat, lp, A, shift,
+                                                                                per_level, round_flag, feats, zsave);
     LAUNCHED();
     return SHACIRA_OK;
 }
 
 template <int C, int F>
 int bwd3d(const float* coords, const int32_t* perm, int64_t n, const float* g, const float* zsave, const LevelParams& lp,
-          const float* A, int per_level, uint32_t skip_mask, uint32_t level_mask, int red_w, float* gl, float* gA,
-          float* gS, cudaStream_t s, int ctas_per_sm) {
+          const float* A, int per_level, uint32_t skip_mask, uint32_t level_mask, float* gl, float* gA, float* gS,
+          cudaStream_t s, int ctas_per_sm) {
     const int nA = per_level ? lp.num_lods : 1;
-    if (!A && (C != F || red_w < 8)) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "3D backward: A is NULL");
-    if (red_w >= 8) {   // lane pairs, persistent CTAs
-        const bool dec = gA != nullptr || gS != nullptr;
-        const size_t smem = LpBwdLayout<C, F>::bytes(lp.num_lods, nA, dec);
-        if (smem > 200 * 1024) return fail(SHACIRA_ERR_UNSUPPORTED, "3D backward: %zu bytes of shared memory per CTA", smem);
-        static unsigned long long configured = 0ull;
-        if (needs_config(configured))
-            CUDA_OK(cudaFuncSetAttribute(latent_bwd3d_lp_kernel<C, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        const char* e_ctas = getenv("SHACIRA_3D_BWD_CTAS");
-        const int per_sm = (e_ctas && atoi(e_ctas) > 0) ? atoi(e_ctas) : ctas_per_sm;
-        int64_t blocks = (n + kLpChunk - 1) / kLpChunk;
-        const int64_t cap = (int64_t)sm_count() * per_sm;
-        if (blocks > cap) blocks = cap;
-        latent_bwd3d_lp_kernel<C, F><<<(int)blocks, kLpBlock, smem, s>>>(coords, perm, n, g, zsave, lp, A, per_level,
-                                                                          skip_mask, level_mask, gl, gA, gS);
-        LAUNCHED();
-        return SHACIRA_OK;
-    }
-    const size_t smem = sizeof(float) * (size_t)(nA * C * F + lp.num_lods * C * F + lp.num_lods * F);
-    latent_bwd3d_kernel<C, F><<<grid_for(n, kBlock), kBlock, smem, s>>>(coords, perm, n, g, zsave, lp, A, per_level,
-                                                                         skip_mask, level_mask, red_w, gl, gA, gS);
+    if (!A && C != F) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "3D backward: A is NULL");
+    const bool dec = gA != nullptr || gS != nullptr;
+    const size_t smem = LpBwdLayout<C, F>::bytes(lp.num_lods, nA, dec);
+    if (smem > 200 * 1024) return fail(SHACIRA_ERR_UNSUPPORTED, "3D backward: %zu bytes of shared memory per CTA", smem);
+    static unsigned long long configured = 0ull;
+    if (needs_config(configured))
+        CUDA_OK(cudaFuncSetAttribute(latent_bwd3d_lp_kernel<C, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    int64_t blocks = (n + kLpChunk - 1) / kLpChunk;   // persistent CTAs
+    const int64_t cap = (int64_t)sm_count() * ctas_per_sm;
+    if (blocks > cap) blocks = cap;
+    latent_bwd3d_lp_kernel<C, F><<<(int)blocks, kLpBlock, smem, s>>>(coords, perm, n, g, zsave, lp, A, per_level,
+                                                                      skip_mask, level_mask, gl, gA, gS);
     LAUNCHED();
     return SHACIRA_OK;
 }
@@ -108,9 +81,9 @@ int launch_fwd3d(int C, int F, const float* coords, const int32_t* perm, int64_t
 
 int launch_bwd3d(int C, int F, const float* coords, const int32_t* perm, int64_t n, const float* grad_out,
                  const float* zsave, const LevelParams& lp, const float* A, int per_level, uint32_t skip_mask,
-                 uint32_t level_mask, int red_w, float* grad_latents, float* grad_A, float* grad_shift, cudaStream_t s,
+                 uint32_t level_mask, float* grad_latents, float* grad_A, float* grad_shift, cudaStream_t s,
                  int ctas_per_sm) {
-    G3_DISPATCH(C, F, (bwd3d<kC, kF>(coords, perm, n, grad_out, zsave, lp, A, per_level, skip_mask, level_mask, red_w,
+    G3_DISPATCH(C, F, (bwd3d<kC, kF>(coords, perm, n, grad_out, zsave, lp, A, per_level, skip_mask, level_mask,
                                      grad_latents, grad_A, grad_shift, s, ctas_per_sm)))
 }
 

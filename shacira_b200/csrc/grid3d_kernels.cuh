@@ -1,405 +1,32 @@
-// grid3d_kernels.cuh -- 3D latent-grid kernels built around the SECTOR economy of the B200 memory system.
+// grid3d_kernels.cuh -- 3D latent-grid kernels built around the REQUEST economy of the B200 memory system.
 //
 // Reference: hashgrid_interpolate_cuda.cu:47-109 (forward) and :143-271 (backward): one thread per point and level,
 // 8 scalar corner gathers / 8 scalar atomicAdds. On the fine levels of a NeRF-shape grid every sample sits in a cell of
-// its own, so nothing is shared between samples and the cost is the number of 32-byte sectors that miss L1 (forward)
-// or of L2 atomic operations (backward) per sample and level (profiles/r01b_ncu_3d_fwd_summary.txt: one sector per
-// 4-byte gather, 31.4 sectors per request, the L1 miss path saturated at ~1 sector / clk / SM).
+// its own, so nothing is shared between samples (profiles/r01b_ncu_3d_fwd_summary.txt: one sector per 4-byte gather,
+// 31.4 sectors per request).
 //
-// What these kernels change: the two corners of a cell that differ in x only are neighbours in the table --
-//   dense  : idx(x+1) = idx(x) + 1
-//   hashed : idx(x) = (x ^ h) & m,  idx(x+1) = ((x+1) ^ h) & m,  h = y*P1 ^ z*P2  =>  idx(x) ^ idx(x+1) = x ^ (x+1)
-//            = 2^(t+1) - 1 (t = trailing ones of x): the same aligned block of 2^(t+1) rows
-// so the pair is fetched with ONE aligned 16-byte load (and, in the backward, added with ONE vector `red.global`)
-// whenever both rows fall into the same aligned quad; the lanes where they do not issue a second scalar access.
-// 4 + ~1 accesses per sample and level instead of 8. Indices, weights, rounding and the order of the interpolation sum
-// are those of common.cuh / hashgrid_kernels.cuh: the forward is bit-identical to latent_fwd_kernel.
+// Lane pairs: TWO lanes per sample, lane parity = the x side of the cell (dx).
+// Measured on the B200 (benchmarks/microbench2.cu, profiles/r02a_microbench2.csv; ncu of an earlier one-lane-per-sample
+// form with merged 16-byte x-pair loads, profiles/r02a_ncu_3d_*.txt): what bounds the 3D path is the number of
+// REQUESTS an SM sends to L2 -- ~1 per clock per SM ("L1: M L1tex2xbar Req Cycles Active" 83 %), one per (instruction,
+// 128-byte line) for loads and stores and one per (instruction, 32-byte sector) for reds -- not bytes, sectors or
+// instructions. Two lanes of ONE instruction that touch the same line (loads) / sector (reds) share a request:
+// 294 G pairs/s for loads and 198 G pairs/s for reds, the rates of single accesses. So lanes 2s and 2s+1 work on sample
+// s of the warp's 16 samples: both locate the cell, lane parity picks x or x+1, and every load / red instruction carries
+// the two x-neighbour corners of 16 samples side by side: 4 requests per sample and level instead of 8, on any
+// alignment of the level in the table. Indices, weights and rounding are those of common.cuh, and the interpolation sum
+// keeps the reference's order: the even lane runs corners 0..3, hands its partial sum to the odd lane (one shuffle),
+// which continues with corners 4..7 -- bit-identical to latent_fwd_kernel.
+// Rows (features, upstream gradients, saved z) move through per-warp shared-memory tiles so that every global access
+// is a full 128-byte line: 2 requests per 256-byte row instead of 16.
 //
 // Samples may be given in the plan's tile-sorted order (`perm` != NULL: coords are the plan's sorted copy, row i of the
 // result belongs to sample perm[i]): neighbouring lanes then share the coarse and middle levels' cache lines in L1.
 #pragma once
 #include "common.cuh"
-#include "hashgrid_kernels.cuh"
 
 namespace shacira {
 
-// cell position, interpolation weights (reference corner order k = dx*4 + dy*2 + dz) and the absolute table rows of
-// the 4 x-pairs: pair j = dy*2 + dz holds corner k = j (x) in a[j] and corner k = j + 4 (x + 1) in b[j]
-struct Pairs3 {
-    int32_t a[4], b[4];
-    float w[8];
-};
-
-__device__ __forceinline__ void pairs3(const double (&t)[3], const LevelParams& lp, int l, Pairs3& o) {
-    const int32_t res = lp.res[l];
-    const float hi = lp.hi[l];
-    const int32_t first = lp.first[l];
-    int32_t p[3];
-    float f[3], g[3];
-#pragma unroll
-    for (int d = 0; d < 3; ++d) locate(t[d], res, hi, p[d], f[d], g[d]);
-    const float gg = __fmul_rn(g[0], g[1]), gf = __fmul_rn(g[0], f[1]);
-    const float fg = __fmul_rn(f[0], g[1]), ff = __fmul_rn(f[0], f[1]);
-    o.w[0] = __fmul_rn(gg, g[2]);
-    o.w[1] = __fmul_rn(gg, f[2]);
-    o.w[2] = __fmul_rn(gf, g[2]);
-    o.w[3] = __fmul_rn(gf, f[2]);
-    o.w[4] = __fmul_rn(fg, g[2]);
-    o.w[5] = __fmul_rn(fg, f[2]);
-    o.w[6] = __fmul_rn(ff, g[2]);
-    o.w[7] = __fmul_rn(ff, f[2]);
-    if ((lp.dense_mask >> l) & 1u) {
-        const int32_t last = lp.rows[l] - 1;   // SURVEY Q4: zero-weight corners stay inside the level
-        const int32_t rr = res * res;
-        const int32_t base = p[0] + p[1] * res + p[2] * rr;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int32_t e = base + ((j >> 1) & 1) * res + (j & 1) * rr;
-            o.a[j] = first + min(e, last);
-            o.b[j] = first + min(e + 1, last);
-        }
-    } else {
-        const uint32_t m = lp.hash_mask;
-        const uint32_t x0 = (uint32_t)p[0], x1 = x0 + 1u;
-        const uint32_t hy0 = (uint32_t)p[1] * kPrimeY, hz0 = (uint32_t)p[2] * kPrimeZ;
-        const uint32_t hy[2] = {hy0, hy0 + kPrimeY};
-        const uint32_t hz[2] = {hz0, hz0 + kPrimeZ};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const uint32_t h = hy[(j >> 1) & 1] ^ hz[j & 1];
-            o.a[j] = first + (int32_t)((x0 ^ h) & m);
-            o.b[j] = first + (int32_t)((x1 ^ h) & m);
-        }
-    }
-}
-
-__device__ __forceinline__ float pick4(const float4& q, int j) {
-    return (j == 0) ? q.x : ((j == 1) ? q.y : ((j == 2) ? q.z : q.w));
-}
-
-// The latent rows of one x-pair (C channels each) from ONE aligned 16-byte load when both rows lie in it.
-// `lat16` is the table viewed as float4 (the table pointer is 16-byte aligned: checked by the launcher).
-template <int C>
-__device__ __forceinline__ void load_pair(const float* __restrict__ latents, int32_t ia, int32_t ib, float (&va)[C],
-                                          float (&vb)[C]) {
-    static_assert(C == 1 || C == 2, "pair merging: one or two channels per row");
-    constexpr int RQ = 4 / C;  // rows per 16-byte quad
-    const int32_t qa = ia / RQ;  // ia >= 0
-    const float4 q = __ldg(reinterpret_cast<const float4*>(latents) + qa);
-    const bool same = (ib / RQ) == qa;
-    if constexpr (C == 1) {
-        va[0] = pick4(q, ia & 3);
-        float other = 0.0f;
-        if (!same) other = __ldg(latents + ib);
-        vb[0] = same ? pick4(q, ib & 3) : other;
-    } else {
-        const bool hi_a = ia & 1, hi_b = ib & 1;
-        va[0] = hi_a ? q.z : q.x;
-        va[1] = hi_a ? q.w : q.y;
-        float2 other = make_float2(0.0f, 0.0f);
-        if (!same) other = __ldg(reinterpret_cast<const float2*>(latents) + ib);
-        vb[0] = same ? (hi_b ? q.z : q.x) : other.x;
-        vb[1] = same ? (hi_b ? q.w : q.y) : other.y;
-    }
-}
-
-// ------------------------------------------------------------------------------------------------------------------
-// forward: q = rint(latent) -> trilinear lerp (C channels) -> A^T z + shift (F channels); all levels in one launch
-// ------------------------------------------------------------------------------------------------------------------
-template <int C, int F>
-__global__ void __launch_bounds__(kBlock)
-latent_fwd3d_kernel(const float* __restrict__ coords, const int32_t* __restrict__ perm, int64_t n,
-                    const float* __restrict__ latents, const __grid_constant__ LevelParams lp,
-                    const float* __restrict__ A, const float* __restrict__ shift, int per_level, int round_flag,
-                    float* __restrict__ feats, float* __restrict__ zsave) {
-    extern __shared__ float s_dec[];  // [nA][C*F] then [nA][F]
-    const int L = lp.num_lods;
-    const int nA = per_level ? L : 1;
-    float* s_A = s_dec;
-    float* s_shift = s_dec + nA * C * F;
-    for (int e = threadIdx.x; e < nA * C * F; e += kBlock) s_A[e] = A[e];
-    for (int e = threadIdx.x; e < nA * F; e += kBlock) s_shift[e] = shift ? shift[e] : 0.0f;
-    __syncthreads();
-    const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
-    if (i >= n) return;
-    double t[3];
-    load_unit_coords<3>(coords, i, t);
-    const int64_t row = perm ? (int64_t)__ldg(perm + i) : i;
-    float* out = feats + row * (int64_t)L * F;
-    // zsave is private to this library's forward / backward pair: rows in the order of `coords` (sorted when planned)
-    float* zout = zsave ? zsave + i * (int64_t)L * C : nullptr;
-    constexpr int G = (F >= 4) ? 1 : 4 / F;   // levels per 16-byte output vector
-    constexpr int GZ = 2 / C;                  // levels per 8-byte z vector (two levels in flight keep the registers in check)
-    constexpr int GG = (G > GZ) ? G : GZ;
-    const bool vec_o = (L * F) % 4 == 0, vec_z = (L * C) % 2 == 0;
-    int l = 0;
-    for (; l + GG <= L; l += GG) {
-        Pairs3 pr[GG];
-        float va[GG][4][C], vb[GG][4][C];
-#pragma unroll
-        for (int q = 0; q < GG; ++q) pairs3(t, lp, l + q, pr[q]);
-#pragma unroll
-        for (int q = 0; q < GG; ++q)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) load_pair<C>(latents, pr[q].a[j], pr[q].b[j], va[q][j], vb[q][j]);
-        float o[GG * F], zz[GG * C];
-#pragma unroll
-        for (int q = 0; q < GG; ++q) {
-            const int la = per_level ? (l + q) : 0;
-#pragma unroll
-            for (int ch = 0; ch < C; ++ch) {
-                float v[8];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    v[j] = round_flag ? rintf(va[q][j][ch]) : va[q][j][ch];
-                    v[j + 4] = round_flag ? rintf(vb[q][j][ch]) : vb[q][j][ch];
-                }
-                // contraction order of the reference build: fma(v0,w0, v1*w1), then k = 2..7
-                float acc = __fmul_rn(v[1], pr[q].w[1]);
-                acc = __fmaf_rn(v[0], pr[q].w[0], acc);
-#pragma unroll
-                for (int k = 2; k < 8; ++k) acc = __fmaf_rn(v[k], pr[q].w[k], acc);
-                zz[q * C + ch] = acc;
-            }
-#pragma unroll
-            for (int jf = 0; jf < F; ++jf) {
-                float acc = s_shift[la * F + jf];
-#pragma unroll
-                for (int ch = 0; ch < C; ++ch) acc = __fmaf_rn(zz[q * C + ch], s_A[(la * C + ch) * F + jf], acc);
-                o[q * F + jf] = acc;
-            }
-        }
-        if (vec_o) {
-#pragma unroll
-            for (int q = 0; q < GG / G; ++q) {
-                float tmp[G * F];
-#pragma unroll
-                for (int e = 0; e < G * F; ++e) tmp[e] = o[q * G * F + e];
-                store_row<G * F>(out + (l + q * G) * F, tmp);
-            }
-        } else {
-#pragma unroll
-            for (int e = 0; e < GG * F; ++e) out[l * F + e] = o[e];
-        }
-        if (zout) {
-            if (vec_z) {
-#pragma unroll
-                for (int q = 0; q < GG / GZ; ++q) {
-                    float tmp[GZ * C];
-#pragma unroll
-                    for (int e = 0; e < GZ * C; ++e) tmp[e] = zz[q * GZ * C + e];
-                    store_row<GZ * C>(zout + (l + q * GZ) * C, tmp);
-                }
-            } else {
-#pragma unroll
-                for (int e = 0; e < GG * C; ++e) zout[l * C + e] = zz[e];
-            }
-        }
-    }
-    for (; l < L; ++l) {  // tail levels
-        Pairs3 pr;
-        pairs3(t, lp, l, pr);
-        const int la = per_level ? l : 0;
-        float zc[C];
-        float va[4][C], vb[4][C];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) load_pair<C>(latents, pr.a[j], pr.b[j], va[j], vb[j]);
-#pragma unroll
-        for (int ch = 0; ch < C; ++ch) {
-            float v[8];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                v[j] = round_flag ? rintf(va[j][ch]) : va[j][ch];
-                v[j + 4] = round_flag ? rintf(vb[j][ch]) : vb[j][ch];
-            }
-            float acc = __fmul_rn(v[1], pr.w[1]);
-            acc = __fmaf_rn(v[0], pr.w[0], acc);
-#pragma unroll
-            for (int k = 2; k < 8; ++k) acc = __fmaf_rn(v[k], pr.w[k], acc);
-            zc[ch] = acc;
-            if (zout) zout[l * C + ch] = acc;
-        }
-        for (int jf = 0; jf < F; ++jf) {
-            float acc = s_shift[la * F + jf];
-#pragma unroll
-            for (int ch = 0; ch < C; ++ch) acc = __fmaf_rn(zc[ch], s_A[(la * C + ch) * F + jf], acc);
-            out[l * F + jf] = acc;
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------------------------------
-// backward: grad_latents[row] += w_k * sum_f g[f] A[c][f]; one vector `red.global` per x-pair when both rows share an
-// aligned quad (zeros ride in the unused lanes: x + 0 = x), else the second row gets a scalar / row-wide red.
-// RED_W: 4 = 16-byte vector reds on the aligned quad, 2 = 8-byte vector reds on the aligned pair (C = 1), 0 = one
-// red per corner (A/B runs). Decoder gradients as in latent_bwd_kernel (warp -> block -> global), from `zsave`.
-// ------------------------------------------------------------------------------------------------------------------
-template <int C>
-__device__ __forceinline__ void red_pair(float* __restrict__ grad, int32_t ia, int32_t ib, const float (&ga)[C],
-                                         const float (&gb)[C], int red_w) {
-    static_assert(C == 1 || C == 2, "pair merging: one or two channels per row");
-    if constexpr (C == 1) {
-        if (red_w == 4) {
-            const int32_t qa = ia >> 2;
-            const bool same = (ib >> 2) == qa;
-            const int ja = ia & 3, jb = ib & 3;
-            float v[4];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) v[j] = ((j == ja) ? ga[0] : 0.0f) + ((same && j == jb) ? gb[0] : 0.0f);
-            red_add4(grad + 4 * (int64_t)qa, v[0], v[1], v[2], v[3]);
-            if (!same) red_add(grad + ib, gb[0]);
-        } else if (red_w == 2) {
-            const int32_t qa = ia >> 1;
-            const bool same = (ib >> 1) == qa;
-            const int ja = ia & 1, jb = ib & 1;
-            float v[2];
-#pragma unroll
-            for (int j = 0; j < 2; ++j) v[j] = ((j == ja) ? ga[0] : 0.0f) + ((same && j == jb) ? gb[0] : 0.0f);
-            red_add2(grad + 2 * (int64_t)qa, v[0], v[1]);
-            if (!same) red_add(grad + ib, gb[0]);
-        } else {
-            red_add(grad + ia, ga[0]);
-            red_add(grad + ib, gb[0]);
-        }
-    } else {
-        if (red_w == 4) {
-            const int32_t qa = ia >> 1;
-            const bool same = (ib >> 1) == qa;
-            const bool hi_a = ia & 1, hi_b = ib & 1;
-            float v[4];
-            v[0] = (hi_a ? 0.0f : ga[0]) + ((same && !hi_b) ? gb[0] : 0.0f);
-            v[1] = (hi_a ? 0.0f : ga[1]) + ((same && !hi_b) ? gb[1] : 0.0f);
-            v[2] = (hi_a ? ga[0] : 0.0f) + ((same && hi_b) ? gb[0] : 0.0f);
-            v[3] = (hi_a ? ga[1] : 0.0f) + ((same && hi_b) ? gb[1] : 0.0f);
-            red_add4(grad + 4 * (int64_t)qa, v[0], v[1], v[2], v[3]);
-            if (!same) red_add2(grad + 2 * (int64_t)ib, gb[0], gb[1]);
-        } else {
-            red_add2(grad + 2 * (int64_t)ia, ga[0], ga[1]);
-            red_add2(grad + 2 * (int64_t)ib, gb[0], gb[1]);
-        }
-    }
-}
-
-template <int C, int F>
-__global__ void __launch_bounds__(kBlock)
-latent_bwd3d_kernel(const float* __restrict__ coords, const int32_t* __restrict__ perm, int64_t n,
-                    const float* __restrict__ grad_out, const float* __restrict__ zsave,
-                    const __grid_constant__ LevelParams lp, const float* __restrict__ A, int per_level,
-                    uint32_t skip_mask, uint32_t level_mask, int red_w, float* __restrict__ grad_latents,
-                    float* __restrict__ grad_A, float* __restrict__ grad_shift) {
-    extern __shared__ float s_mem[];  // A [nA*C*F] | gA [L*C*F] | gS [L*F]
-    const int L = lp.num_lods;
-    const int nA = per_level ? L : 1;
-    float* s_A = s_mem;
-    float* s_gA = s_A + nA * C * F;
-    float* s_gS = s_gA + L * C * F;
-    for (int e = threadIdx.x; e < nA * C * F; e += kBlock) s_A[e] = A[e];
-    for (int e = threadIdx.x; e < L * C * F + L * F; e += kBlock) s_gA[e] = 0.0f;
-    __syncthreads();
-    const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
-    const bool live = i < n;
-    const bool want_dec = (grad_A != nullptr) || (grad_shift != nullptr);
-    const int lane = threadIdx.x & 31;
-    double t[3];
-    int64_t row = i;
-    if (live) {
-        load_unit_coords<3>(coords, i, t);
-        if (perm) row = __ldg(perm + i);
-    }
-    const float* g_row = grad_out + row * (int64_t)L * F;
-    const float* z_row = zsave ? zsave + i * (int64_t)L * C : nullptr;   // rows in the order of `coords`
-    const bool vec_g = (F == 1) || ((L * F) % (F >= 4 ? 4 : F) == 0);
-    const bool vec_z = (C == 1) || ((L * C) % (C >= 4 ? 4 : C) == 0);
-#pragma unroll 2
-    for (int l = 0; l < L; ++l) {
-        if (!((level_mask >> l) & 1u)) continue;
-        const bool scatter = !((skip_mask >> l) & 1u);
-        if (!scatter && !want_dec) continue;
-        float g[F];
-#pragma unroll
-        for (int j = 0; j < F; ++j) g[j] = 0.0f;
-        if (live) {
-            if (vec_g) {
-                load_row<F>(g_row + l * F, g);
-            } else {
-#pragma unroll
-                for (int j = 0; j < F; ++j) g[j] = __ldg(g_row + l * F + j);
-            }
-        }
-        if (live && scatter) {
-            Pairs3 pr;
-            pairs3(t, lp, l, pr);
-            const int la = per_level ? l : 0;
-            float gz[C];
-#pragma unroll
-            for (int ch = 0; ch < C; ++ch) {
-                float acc = 0.0f;
-#pragma unroll
-                for (int j = 0; j < F; ++j) acc = __fmaf_rn(g[j], s_A[(la * C + ch) * F + j], acc);
-                gz[ch] = acc;
-            }
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                float ga[C], gb[C];
-#pragma unroll
-                for (int ch = 0; ch < C; ++ch) {
-                    ga[ch] = __fmul_rn(gz[ch], pr.w[j]);
-                    gb[ch] = __fmul_rn(gz[ch], pr.w[j + 4]);
-                }
-                red_pair<C>(grad_latents, pr.a[j], pr.b[j], ga, gb, red_w);
-            }
-        }
-        if (want_dec) {  // uniform across the block
-            float z[C];
-#pragma unroll
-            for (int ch = 0; ch < C; ++ch) z[ch] = 0.0f;
-            if (live && z_row) {
-                if (vec_z) {
-                    load_row<C>(z_row + l * C, z);
-                } else {
-#pragma unroll
-                    for (int ch = 0; ch < C; ++ch) z[ch] = __ldg(z_row + l * C + ch);
-                }
-            }
-#pragma unroll
-            for (int j = 0; j < F; ++j) {
-                const float sg = warp_sum(g[j]);
-                if (lane == 0) atomicAdd(&s_gS[l * F + j], sg);
-#pragma unroll
-                for (int ch = 0; ch < C; ++ch) {
-                    const float sa = warp_sum(z[ch] * g[j]);
-                    if (lane == 0) atomicAdd(&s_gA[(l * C + ch) * F + j], sa);
-                }
-            }
-        }
-    }
-    if (want_dec) {
-        __syncthreads();
-        if (grad_A)
-            for (int e = threadIdx.x; e < L * C * F; e += kBlock) red_add(grad_A + e, s_gA[e]);
-        if (grad_shift)
-            for (int e = threadIdx.x; e < L * F; e += kBlock) red_add(grad_shift + e, s_gS[e]);
-    }
-}
-
-
-
-// ==================================================================================================================
-// Lane-pair kernels: TWO lanes per sample, lane parity = the x side of the cell (dx).
-//
-// Measured on the B200 (benchmarks/microbench2.cu, profiles/r02a_microbench2.csv; ncu of the kernels above,
-// profiles/r02a_ncu_3d_*.txt): what bounds the 3D path is the number of REQUESTS an SM sends to L2 -- ~1 per clock
-// per SM ("L1: M L1tex2xbar Req Cycles Active" 83 %), one per (instruction, 128-byte line) for loads and stores and
-// one per (instruction, 32-byte sector) for reds -- not bytes, sectors or instructions. Two lanes of ONE instruction
-// that touch the same line (loads) / sector (reds) share a request: 294 G pairs/s for loads and 198 G pairs/s for
-// reds, the rates of single accesses. So lanes 2s and 2s+1 work on sample s of the warp's 16 samples: both locate
-// the cell, lane parity picks x or x+1, and every load / red instruction carries the two x-neighbour corners of 16
-// samples side by side: 4 requests per sample and level instead of 8, on any alignment of the level in the table.
-// The interpolation sum keeps the reference's order: the even lane runs corners 0..3, hands its partial sum to the odd
-// lane (one shuffle), which continues with corners 4..7 -- bit-identical to latent_fwd_kernel.
-// Rows (features, upstream gradients, saved z) move through per-warp shared-memory tiles so that every global access
-// is a full 128-byte line: 2 requests per 256-byte row instead of 16.
-// ==================================================================================================================
 constexpr int kLpWarps = 8;                  // warps per CTA
 constexpr int kLpBlock = kLpWarps * 32;
 constexpr int kLpSamples = 16;               // samples per warp pass

@@ -15,16 +15,8 @@
 // memory, each lane accumulating an 8-wide slice in registers across ALL its warp's points (persistent CTAs),
 // then reduced over the block in shared memory and added to global memory once per CTA and value.
 #pragma once
-#include <utility>
-
 #include "common.cuh"
 #include "mlp_tc_common.cuh"
-
-// Decoder-MLP weights of the IN = 16 fast path, packed W1 | b1 | W2 | b2 | W3 | b3. C linkage: the kernel names the
-// symbol in inline PTX (see cweight below).
-extern "C" {
-__constant__ float shacira_c_mlp[16 * 16 + 16 + 16 * 16 + 16 + 3 * 16 + 3 + 1];
-}
 
 namespace shacira {
 
@@ -270,259 +262,6 @@ mlp_mse_step_kernel(const float* __restrict__ x, const float* __restrict__ gt, i
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// IN = 16 fast path (the image decoder: 16 levels x 1 feature).
-//
-// The kernel above feeds every FMA of the forward / backward products with a weight broadcast from shared memory
-// (one LDS.128 per 4 FMAs): measured on B200 it is bound by the shared-memory pipe, 82 us at the Kodak shape against
-// an 18 us FP32 floor. Here the 595 weights live in CONSTANT memory (copied device-to-device before the launch), so
-// the products are plain `FFMA R, R, c[bank][imm], R` with no load at all, and the weight-gradient stage splits each
-// warp into two half-warps that walk the even / odd points of the warp's 32: every lane owns a 4 x 4 block of dW1
-// and dW2 (16 FMAs per two 16-byte shared loads instead of 8 per three). Activations are staged unpadded with an XOR
-// swizzle of the 16-byte chunks (conflict-free both for the per-lane row stores and the half-warp block loads).
-// One MLP step may be in flight per device at a time (the constant bank is shared by all streams).
-// ---------------------------------------------------------------------------------------------------------------
-constexpr int kMlpConstFloats = 16 * 16 + 16 + 16 * 16 + 16 + 3 * 16 + 3;  // W1 | b1 | W2 | b2 | W3 | b3 (packed order)
-
-// Weight OFF as an FFMA constant-bank operand (`FFMA R, R, c[3][imm], R`: no load instruction at all). Two things
-// defeat that if the products are written inline in the persistent point loop (both measured with cuobjdump): the
-// 595 loads are loop invariant, so ptxas hoists them into registers and spills 2 KB per thread; and a weight used by
-// the forward AND the backward product becomes one load with two uses, i.e. a register again. Hence the forward and
-// the backward live in two __noinline__ functions: no loop to hoist out of, one use per weight and function.
-template <int OFF>
-__device__ __forceinline__ float cweight() {
-    float w;
-    asm("ld.const.f32 %0, [shacira_c_mlp+%1];" : "=f"(w) : "n"(OFF * 4));
-    return w;
-}
-template <int... Is, class Fn>
-__device__ __forceinline__ void static_for_impl(std::integer_sequence<int, Is...>, Fn&& f) {
-    (f(std::integral_constant<int, Is>{}), ...);
-}
-template <int N, class Fn>
-__device__ __forceinline__ void static_for(Fn&& f) {
-    static_for_impl(std::make_integer_sequence<int, N>{}, f);
-}
-
-struct Mlp16Smem {
-    // per warp: 32 points x 16 floats each, chunk-swizzled; dy padded to 4
-    float x[kMlpWarps][32][16], h1[kMlpWarps][32][16], h2[kMlpWarps][32][16];
-    float d1[kMlpWarps][32][16], d2[kMlpWarps][32][16], dy[kMlpWarps][32][4];
-    uint2 mask[kMlpWarps][32];  // ReLU masks of layers 1 and 2, forward -> backward
-    float g[kMlpConstFloats + 1];  // block reduction of the gradient slices (packed order)
-    double loss;
-};
-
-// physical 16-byte chunk of logical chunk c in row p: the row's parity picks the bank half (row stride 64 B), the
-// rotation by (p >> 1) spreads a quarter-warp's stores over all 32 banks
-__device__ __forceinline__ int swz16(int p, int c) { return c ^ ((p >> 1) & 3); }
-
-namespace mlp16 {
-constexpr int IN = 16, H = 16, OUT = 3;
-constexpr int oW1 = 0, ob1 = oW1 + H * IN, oW2 = ob1 + H, ob2 = oW2 + H * H, oW3 = ob2 + H, ob3 = oW3 + OUT * H;
-}  // namespace mlp16
-
-// Forward of one point per lane: stages x, h1, h2, dy and the ReLU masks of the lane's row; returns its squared error.
-__device__ __noinline__ float mlp16_forward(const float* __restrict__ x, const float* __restrict__ gt, int64_t p,
-                                            int live, float grad_scale, float* __restrict__ pred, Mlp16Smem* Sp,
-                                            int warp, int lane) {
-    using namespace mlp16;
-    Mlp16Smem& S = *Sp;
-    float4* sx = reinterpret_cast<float4*>(&S.x[warp][0][0]);
-    float4* sh1 = reinterpret_cast<float4*>(&S.h1[warp][0][0]);
-    float4* sh2 = reinterpret_cast<float4*>(&S.h2[warp][0][0]);
-    float v[16], h[16], tgt[OUT] = {0.0f, 0.0f, 0.0f};
-#pragma unroll
-    for (int e = 0; e < 16; ++e) v[e] = 0.0f;
-    if (live) {
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const float4 t4 = __ldg(reinterpret_cast<const float4*>(x + p * IN) + q);
-            v[4 * q] = t4.x; v[4 * q + 1] = t4.y; v[4 * q + 2] = t4.z; v[4 * q + 3] = t4.w;
-        }
-#pragma unroll
-        for (int k = 0; k < OUT; ++k) tgt[k] = __ldg(gt + p * OUT + k);
-    }
-#pragma unroll
-    for (int q = 0; q < 4; ++q) sx[lane * 4 + swz16(lane, q)] = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-    unsigned m1 = 0u, m2 = 0u;
-    static_for<H>([&](auto I) {
-        constexpr int i = decltype(I)::value;
-        float acc = cweight<ob1 + i>();
-        static_for<IN>([&](auto M) {
-            constexpr int m = decltype(M)::value;
-            acc = fmaf(v[m], cweight<oW1 + i * IN + m>(), acc);
-        });
-        h[i] = fmaxf(acc, 0.0f);
-        m1 |= (acc > 0.0f ? 1u : 0u) << i;
-    });
-#pragma unroll
-    for (int q = 0; q < 4; ++q) sh1[lane * 4 + swz16(lane, q)] = make_float4(h[4 * q], h[4 * q + 1], h[4 * q + 2], h[4 * q + 3]);
-    static_for<H>([&](auto J) {
-        constexpr int j = decltype(J)::value;
-        float acc = cweight<ob2 + j>();
-        static_for<H>([&](auto I) {
-            constexpr int i = decltype(I)::value;
-            acc = fmaf(h[i], cweight<oW2 + j * H + i>(), acc);
-        });
-        v[j] = fmaxf(acc, 0.0f);   // v now holds h2
-        m2 |= (acc > 0.0f ? 1u : 0u) << j;
-    });
-#pragma unroll
-    for (int q = 0; q < 4; ++q) sh2[lane * 4 + swz16(lane, q)] = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-    float dy[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-    float loss = 0.0f;
-    static_for<OUT>([&](auto K) {
-        constexpr int k = decltype(K)::value;
-        float acc = cweight<ob3 + k>();
-        static_for<H>([&](auto J) {
-            constexpr int j = decltype(J)::value;
-            acc = fmaf(v[j], cweight<oW3 + k * H + j>(), acc);
-        });
-        if (live) {
-            const float e = acc - tgt[k];
-            loss = fmaf(e, e, loss);
-            dy[k] = e * grad_scale;
-            if (pred) pred[p * OUT + k] = acc;
-        }
-    });
-    reinterpret_cast<float4*>(&S.dy[warp][0][0])[lane] = make_float4(dy[0], dy[1], dy[2], dy[3]);
-    S.mask[warp][lane] = make_uint2(m1, m2);
-    return loss;
-}
-
-// Backward of the lane's point: d2, d1 (staged) and the feature gradient row.
-__device__ __noinline__ void mlp16_backward(int64_t p, int live, float* __restrict__ gx, Mlp16Smem* Sp, int warp,
-                                            int lane) {
-    using namespace mlp16;
-    Mlp16Smem& S = *Sp;
-    float4* sd1 = reinterpret_cast<float4*>(&S.d1[warp][0][0]);
-    float4* sd2 = reinterpret_cast<float4*>(&S.d2[warp][0][0]);
-    const float4 dy4 = reinterpret_cast<const float4*>(&S.dy[warp][0][0])[lane];
-    const uint2 mk = S.mask[warp][lane];
-    const float dy[3] = {dy4.x, dy4.y, dy4.z};
-    float h[16], v[16];
-    static_for<H>([&](auto J) {   // d2 -> h[]
-        constexpr int j = decltype(J)::value;
-        float acc = dy[0] * cweight<oW3 + j>();
-        acc = fmaf(dy[1], cweight<oW3 + H + j>(), acc);
-        acc = fmaf(dy[2], cweight<oW3 + 2 * H + j>(), acc);
-        h[j] = ((mk.y >> j) & 1u) ? acc : 0.0f;
-    });
-#pragma unroll
-    for (int q = 0; q < 4; ++q) sd2[lane * 4 + swz16(lane, q)] = make_float4(h[4 * q], h[4 * q + 1], h[4 * q + 2], h[4 * q + 3]);
-    static_for<H>([&](auto I) {   // d1 -> v[]
-        constexpr int i = decltype(I)::value;
-        float acc = 0.0f;
-        static_for<H>([&](auto J) {
-            constexpr int j = decltype(J)::value;
-            acc = fmaf(h[j], cweight<oW2 + j * H + i>(), acc);
-        });
-        v[i] = ((mk.x >> i) & 1u) ? acc : 0.0f;
-    });
-#pragma unroll
-    for (int q = 0; q < 4; ++q) sd1[lane * 4 + swz16(lane, q)] = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-    if (live) {
-        float o[IN];
-        static_for<IN>([&](auto M) {
-            constexpr int m = decltype(M)::value;
-            float acc = 0.0f;
-            static_for<H>([&](auto I) {
-                constexpr int i = decltype(I)::value;
-                acc = fmaf(v[i], cweight<oW1 + i * IN + m>(), acc);
-            });
-            o[m] = acc;
-        });
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-            reinterpret_cast<float4*>(gx + p * IN)[q] = make_float4(o[4 * q], o[4 * q + 1], o[4 * q + 2], o[4 * q + 3]);
-    }
-}
-
-__global__ void __launch_bounds__(kMlpThreads, 2)
-mlp16_mse_step_kernel(const float* __restrict__ x, const float* __restrict__ gt, int64_t n, float grad_scale,
-                      float* __restrict__ gx, float* __restrict__ pred, double* __restrict__ loss_sum,
-                      float* __restrict__ grad_params) {
-    using namespace mlp16;
-    extern __shared__ __align__(16) unsigned char s_raw[];
-    Mlp16Smem& S = *reinterpret_cast<Mlp16Smem*>(s_raw);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    for (int e = tid; e < kMlpConstFloats + 1; e += kMlpThreads) S.g[e] = 0.0f;
-    if (tid == 0) S.loss = 0.0;
-    __syncthreads();
-    // weight-gradient ownership: half = lane >> 4 walks points of that parity; r = lane & 15 -> block (ib, jb)
-    const int half = lane >> 4, r = lane & 15, ib = r >> 2, jb = r & 3;
-    float aW1[4][4], aW2[4][4], aW3[4], ab1[4], ab2[4], ab3 = 0.0f;
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-        aW3[a] = 0.0f; ab1[a] = 0.0f; ab2[a] = 0.0f;
-#pragma unroll
-        for (int b = 0; b < 4; ++b) { aW1[a][b] = 0.0f; aW2[a][b] = 0.0f; }
-    }
-    float my_loss = 0.0f;
-    float4* sx = reinterpret_cast<float4*>(&S.x[warp][0][0]);
-    float4* sh1 = reinterpret_cast<float4*>(&S.h1[warp][0][0]);
-    float4* sh2 = reinterpret_cast<float4*>(&S.h2[warp][0][0]);
-    float4* sd1 = reinterpret_cast<float4*>(&S.d1[warp][0][0]);
-    float4* sd2 = reinterpret_cast<float4*>(&S.d2[warp][0][0]);
-
-    const int64_t warps_total = (int64_t)gridDim.x * kMlpWarps;
-    for (int64_t base = ((int64_t)blockIdx.x * kMlpWarps + warp) * 32; base < n; base += warps_total * 32) {
-        const int64_t p = base + lane;
-        const int live = p < n;
-        __syncwarp();  // the previous iteration's weight-gradient reads of the staging rows are done
-        my_loss += mlp16_forward(x, gt, p, live, grad_scale, pred, &S, warp, lane);
-        mlp16_backward(p, live, gx, &S, warp, lane);
-        __syncwarp();
-        // ---- weight gradients: this half-warp walks the points of its parity ----
-#pragma unroll 4
-        for (int t = 0; t < 16; ++t) {
-            const int q = 2 * t + half;
-            const float4 d1v = sd1[q * 4 + swz16(q, ib)];   // d1[q][4 ib ..]
-            const float4 xv = sx[q * 4 + swz16(q, jb)];     // x[q][4 jb ..]
-            const float4 d2v = sd2[q * 4 + swz16(q, ib)];
-            const float4 h1v = sh1[q * 4 + swz16(q, jb)];
-            const float4 h2v = sh2[q * 4 + swz16(q, jb)];
-            const float dyk = S.dy[warp][q][ib];            // ib doubles as the output index k (3 is the zero pad)
-            const float a1[4] = {d1v.x, d1v.y, d1v.z, d1v.w}, bx[4] = {xv.x, xv.y, xv.z, xv.w};
-            const float a2[4] = {d2v.x, d2v.y, d2v.z, d2v.w}, bh[4] = {h1v.x, h1v.y, h1v.z, h1v.w};
-            const float b3v[4] = {h2v.x, h2v.y, h2v.z, h2v.w};
-#pragma unroll
-            for (int a = 0; a < 4; ++a) {
-#pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    aW1[a][b] = fmaf(a1[a], bx[b], aW1[a][b]);
-                    aW2[a][b] = fmaf(a2[a], bh[b], aW2[a][b]);
-                }
-                ab1[a] += a1[a];      // only the jb == 0 lanes' copies are used
-                ab2[a] += a2[a];
-                aW3[a] = fmaf(dyk, b3v[a], aW3[a]);
-            }
-            ab3 += dyk;
-        }
-    }
-    // ---- block reduction in shared memory, then one global add per CTA and value ----
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-#pragma unroll
-        for (int b = 0; b < 4; ++b) {
-            atomicAdd(&S.g[oW1 + (4 * ib + a) * IN + 4 * jb + b], aW1[a][b]);
-            atomicAdd(&S.g[oW2 + (4 * ib + a) * H + 4 * jb + b], aW2[a][b]);
-        }
-        if (ib < OUT) atomicAdd(&S.g[oW3 + ib * H + 4 * jb + a], aW3[a]);
-        if (jb == 0) {
-            atomicAdd(&S.g[ob1 + 4 * ib + a], ab1[a]);
-            atomicAdd(&S.g[ob2 + 4 * ib + a], ab2[a]);
-        }
-    }
-    if (jb == 0 && ib < OUT) atomicAdd(&S.g[ob3 + ib], ab3);
-    const float wl = warp_sum(my_loss);
-    if (lane == 0) atomicAdd(&S.loss, (double)wl);
-    __syncthreads();
-    for (int e = tid; e < kMlpConstFloats; e += kMlpThreads) red_add(grad_params + e, S.g[e]);
-    if (tid == 0) atomicAdd(loss_sum, S.loss);
-}
-
-// ---------------------------------------------------------------------------------------------------------------
 // IN = 16 on the tensor cores: mma.sync m16n8k8 TF32 with 3xTF32 error compensation.
 //
 // Every product of the step is a small dense contraction -- forward [32 points x 16] x [16 x 16], backward the same
@@ -539,9 +278,12 @@ mlp16_mse_step_kernel(const float* __restrict__ x, const float* __restrict__ gt,
 // Weight gradients need the point index as K: the activations are staged per warp in shared memory ([point][24],
 // conflict-free for both the fragment-layout stores and the transposed fragment loads).
 // ---------------------------------------------------------------------------------------------------------------
+constexpr int kMlp16Params = 16 * 16 + 16 + 16 * 16 + 16 + 3 * 16 + 3;  // W1 | b1 | W2 | b2 | W3 | b3 (packed order)
+
 // MT = m16 tiles (16 points each) a warp runs per iteration; WARPS per CTA. MT = 2 halves the per-point overhead
 // (weight-fragment loads, loop control); MT = 1 halves the registers and the staging rows, i.e. doubles the warps
-// an SM can hold. Both are built; the launcher picks (SHACIRA_MLP_MT, default chosen by measurement).
+// an SM can hold. The launcher builds MT = 2 with 6 warps x 2 CTAs per SM: measured against MT = 1 (6 warps x 3 CTAs,
+// 8 warps x 2 CTAs), which was then removed.
 template <int MT, int WARPS>
 struct MlpTcSmem {
     uint4 wf[20][32];                       // weight fragments (see the enum in the kernel)
@@ -549,7 +291,7 @@ struct MlpTcSmem {
     float x[WARPS][16 * MT][kTcStride], h1[WARPS][16 * MT][kTcStride], h2[WARPS][16 * MT][kTcStride];
     float d1[WARPS][16 * MT][kTcStride], d2[WARPS][16 * MT][kTcStride];
     float dy[WARPS][16 * MT][8];
-    float g[kMlpConstFloats + 1];           // block reduction of the gradients (packed order)
+    float g[kMlp16Params + 1];              // block reduction of the gradients (packed order)
     unsigned cmax[16];                      // max |feature gradient| per input column (bit patterns)
     double loss;
 };
@@ -571,7 +313,7 @@ mlp16_tc_step_kernel(const float* __restrict__ x, const float* __restrict__ gt, 
     Smem& S = *reinterpret_cast<Smem*>(s_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
     tc_build_fragments(S.wf, W1, W2, W3, tid, kTcThreads);
-    for (int e = tid; e < kMlpConstFloats + 1; e += kTcThreads) S.g[e] = 0.0f;
+    for (int e = tid; e < kMlp16Params + 1; e += kTcThreads) S.g[e] = 0.0f;
     if (tid < H) { S.b1[tid] = b1[tid]; S.b2[tid] = b2[tid]; }
     if (tid < 4) S.b3[tid] = tid < OUT ? b3[tid] : 0.0f;
     if (tid == 0) S.loss = 0.0;
@@ -806,7 +548,7 @@ mlp16_tc_step_kernel(const float* __restrict__ x, const float* __restrict__ gt, 
     const float wl = warp_sum(my_loss);
     if (lane == 0) atomicAdd(&S.loss, (double)wl);
     __syncthreads();
-    for (int e = tid; e < kMlpConstFloats; e += kTcThreads) red_add(grad_params + e, S.g[e]);
+    for (int e = tid; e < kMlp16Params; e += kTcThreads) red_add(grad_params + e, S.g[e]);
     if (gx_absmax && tid < 16) atomicMax(gx_absmax + tid, S.cmax[tid]);
     if (tid == 0) atomicAdd(loss_sum, S.loss);
 }

@@ -1,7 +1,5 @@
 // peer_capi.cu -- extern "C" entry points of the peer-memory exchange step (declared in include/shacira_b200.h):
 // allocation / CUDA-IPC export / mapping of the gradient arenas and the one-kernel all-reduce over NVLink.
-#include <cstdlib>
-
 #include "capi_internal.h"
 #include "peer_kernels.cuh"
 
@@ -10,6 +8,7 @@ using namespace shacira;
 namespace {
 
 size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+constexpr int kPeerBlocksPerSm = 2;   // persistent CTAs of the exchange kernels
 
 int fill_view(PeerView& v, void* const* bufs, int64_t flags_offset, int rank, int world) {
     if (world < 2 || world > kPeerMax || (world & (world - 1)))
@@ -30,8 +29,7 @@ template <bool ADAM>
 int launch_peer(const PeerView& v, int64_t numel4, const PeerAdam& ad, cudaStream_t s) {
     const int64_t per = (numel4 + v.world - 1) / v.world;
     int64_t blocks = (per + kPeerThreads - 1) / kPeerThreads;
-    static const int per_sm = [] { const char* e = getenv("SHACIRA_PEER_BLOCKS_PER_SM"); int k = e ? atoi(e) : 0; return k > 0 ? k : 2; }();
-    const int64_t cap = (int64_t)sm_count() * per_sm;
+    const int64_t cap = (int64_t)sm_count() * kPeerBlocksPerSm;
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
     switch (v.world) {
@@ -150,8 +148,7 @@ int shacira_peer_allreduce_multimem(void* multicast_ptr, void* const* flag_bufs,
     const int64_t numel4 = numel / 4;
     const int64_t per = (numel4 + world - 1) / world;
     int64_t blocks = (per + kPeerThreads * 4 - 1) / (kPeerThreads * 4);
-    static const int per_sm = [] { const char* e = getenv("SHACIRA_PEER_BLOCKS_PER_SM"); int k = e ? atoi(e) : 0; return k > 0 ? k : 2; }();
-    const int64_t cap = (int64_t)sm_count() * per_sm;
+    const int64_t cap = (int64_t)sm_count() * kPeerBlocksPerSm;
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
     cudaStream_t s = (cudaStream_t)stream;

@@ -39,13 +39,6 @@ int smem_budget() {
     return b;
 }
 
-// experiment knob: pad the dynamic shared memory so that fewer CTAs are resident per SM
-size_t smem_pad(size_t smem) {
-    const char* env = getenv("SHACIRA_TILE_SMEM_TOTAL");
-    const size_t want = env ? (size_t)atoi(env) : 0;
-    return (want > smem && want <= 48 * 1024) ? want : smem;
-}
-
 PlanView view_of(const shacira_plan* p) {
     PlanView v;
     v.perm = p->sorted_io ? nullptr : p->perm;
@@ -114,12 +107,10 @@ int launch_fwd(shacira_plan* p, const float* lat, const LevelParams& lp, const f
     if (rc_tab) return rc_tab;
     size_t smem = sizeof(float) * ((size_t)cap * C + nA * C * F + nA * F);
     // scattered rows (original point order) of 16..64 floats: collected per batch in shared memory and written as whole rows
-    static const int rows_knob = [] { const char* e = getenv("SHACIRA_FWD_ROWS_SMEM"); return e ? atoi(e) : 1; }();
     const int RL = lp.num_lods * F;
     const size_t rows_bytes = ((smem + 15) & ~(size_t)15) - smem + sizeof(float) * (size_t)kTileThreads * kPts * (RL + 4 + 1);
-    const int rows_via_smem = rows_knob && !p->sorted_io && RL % 4 == 0 && RL <= 64 && smem + rows_bytes <= 46 * 1024;
+    const int rows_via_smem = !p->sorted_io && RL % 4 == 0 && RL <= 64 && smem + rows_bytes <= 46 * 1024;
     if (rows_via_smem) smem += rows_bytes;
-    smem = smem_pad(smem);
     latent_fwd_tiled_kernel<D, C, F><<<p->ntiles, kTileThreads, smem, s>>>(view_of(p), lat, lp, A, shift, per_level,
                                                                             round_flag, feats, cap, rows_via_smem);
     LAUNCHED();
@@ -145,7 +136,6 @@ int launch_bwd(shacira_plan* p, const float* g, const float* lat, const LevelPar
     constexpr int NW = kTileThreads / 32;
     size_t smem = sizeof(float) * ((size_t)cap_acc * CA + (dec ? (size_t)cap * C : 0) + nA * C * F);
     if (dec) smem += sizeof(float) * (size_t)(zp ? NW : 1) * lp.num_lods * (C * F + F);
-    smem = smem_pad(smem);
     if (dec)
         latent_bwd_tiled_kernel<D, C, F, true><<<p->ntiles, kTileThreads, smem, s>>>(view_of(p), g, lat, lp, A, per_level,
                                                                                       round_flag, gl, gA, gS, cap, cap_acc, level_max, SHACIRA_MAX_LEVELS, 0);
@@ -156,20 +146,18 @@ int launch_bwd(shacira_plan* p, const float* g, const float* lat, const LevelPar
     return SHACIRA_OK;
 }
 
-// ---- 3D (NeRF samples): sorted point-parallel kernels with merged x-pair accesses + tile-staged coarse levels ------
+// ---- 3D (NeRF samples): lane-pair kernels on the sorted samples + tile-staged coarse levels ------------------------
 // Number of leading levels the tiled backward stages in shared memory for this plan: while the (upper bound of the)
 // node box of a tile stays below the corner touches of an average tile (otherwise staging only adds a flush) and
-// the boxes fit the shared-memory budget. SHACIRA_3D_STAGED overrides (0 = none).
+// the boxes fit the shared-memory budget.
 int staged_prefix_3d(const shacira_plan* p, const LevelParams& lp, int cap_max, int* cap_out) {
-    const char* env = getenv("SHACIRA_3D_STAGED");
-    const int forced = env ? atoi(env) : -1;
     const double touches = 8.0 * (double)p->n / (double)p->ntiles;
     long long run = 0;
     int ns = 0;
     for (int l = 0; l < lp.num_lods; ++l) {
         const long long w = lp.res[l] / p->g + 3, nodes = w * w * w;
         if (run + nodes > cap_max) break;
-        if (forced >= 0 ? l >= forced : (double)nodes > touches) break;
+        if ((double)nodes > touches) break;
         run += nodes;
         ++ns;
     }
@@ -202,7 +190,6 @@ int launch_bwd_staged3d(shacira_plan* p, const float* g, const LevelParams& lp, 
 int backward_3d_two(shacira_plan* p, const float* g, const float* zsave, const LevelParams& lp, int C, int F, const float* A,
                     int per_level, float* gl, float* gA, float* gS, int ns, int cap, cudaStream_t s) {
     const uint32_t skip = ns >= 32 ? 0xffffffffu : ((1u << ns) - 1u);
-    const int red_w = grid3d_red_mode() < 0 ? 0 : grid3d_red_mode();
     SideStream* ss = nullptr;
     if (ns > 0) {
         if (int rc = side_stream(&ss)) return rc;
@@ -213,7 +200,7 @@ int backward_3d_two(shacira_plan* p, const float* g, const float* zsave, const L
     // staged kernel runs beside it), the tile-staged kernel by shared memory and issue slots; launched in this
     // order the two share every SM instead of queueing behind each other's CTAs.
     int rc = launch_bwd3d(C, F, p->coords_sorted, p->sorted_io ? nullptr : p->perm, p->n, g, zsave, lp, A, per_level, skip,
-                          0xffffffffu, red_w, gl, gA, gS, s, ns > 0 ? 2 : 4);
+                          0xffffffffu, gl, gA, gS, s, ns > 0 ? 2 : 4);
     if (rc) return rc;
     bool forked = false;
     if (ns > 0) {
@@ -245,7 +232,7 @@ int backward_3d(shacira_plan* p, const float* g, const float* zsave, const Level
     int cap = 32;
     const int budget = smem_budget();
     const int rep = (kRepBudget / C) & ~3;
-    const int ns = (grid3d_red_mode() >= 0) ? staged_prefix_3d(p, lp, (budget - rep * 4 * C) / (4 * C), &cap) : 0;
+    const int ns = staged_prefix_3d(p, lp, (budget - rep * 4 * C) / (4 * C), &cap);
     if (!num_lods_ok(lp)) cap = 32;
     const int ns_two = num_lods_ok(lp) ? ns : 0;   // the two-kernel form: the tiled kernel unrolls 4 levels
     return backward_3d_two(p, g, zsave, lp, C, F, A, per_level, gl, gA, gS, ns_two, cap, s);
@@ -275,10 +262,7 @@ int choose_tiles_per_axis(int dim, int64_t n, int tile_points) {
     if (tile_points <= 0) {
         // 2D: ~384 points per tile (tuned round 1). 3D: ~128 samples, i.e. 16 tiles per axis at the NeRF batch: the
         // middle levels' node boxes stay small enough to live in L1 / shared memory (profiles/r02b_probe3d.jsonl)
-        const char* env = getenv(dim == 3 ? "SHACIRA_TILE_POINTS_3D" : "SHACIRA_TILE_POINTS");
-        const int dflt = dim == 3 ? 128 : 384;
-        tile_points = env ? atoi(env) : dflt;
-        if (tile_points <= 0) tile_points = dflt;
+        tile_points = dim == 3 ? 128 : 384;
     }
     // power of two per axis, about tile_points points per tile, at most kMaxTiles tiles
     int g = 1;
@@ -424,7 +408,7 @@ int shacira_latent_forward_planned(const shacira_plan_t* plan, const float* late
     if (rc) return rc;
     if (!latents || !feats || !A) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "latents/feats/A is NULL");
     cudaStream_t s = (cudaStream_t)stream;
-    if (plan->dim == 3 && grid3d_merge_mode() > 0 && grid3d_supported(latent_dim, feature_dim, latents))
+    if (plan->dim == 3 && grid3d_supported(latent_dim, feature_dim, latents))
         return launch_fwd3d(latent_dim, feature_dim, plan->coords_sorted, plan->sorted_io ? nullptr : plan->perm, plan->n,
                             latents, lp, A, shift, per_level, round_flag, feats, nullptr, s);
     if (num_lods % 4) return fail(SHACIRA_ERR_UNSUPPORTED, "the tiled path needs num_lods %% 4 == 0 (got %d)", num_lods);
@@ -453,8 +437,7 @@ int shacira_latent_backward_planned_bounded(const shacira_plan_t* plan, const fl
     if (latent_dim != 1 && latent_dim != 2 && latent_dim != 4)
         return fail(SHACIRA_ERR_UNSUPPORTED, "latent_dim %d not in {1,2,4}", latent_dim);
     cudaStream_t s = (cudaStream_t)stream;
-    if (plan->dim == 3 && !grad_A && !grad_shift && grid3d_red_mode() >= 0 &&
-        grid3d_supported(latent_dim, feature_dim, grad_latents)) {
+    if (plan->dim == 3 && !grad_A && !grad_shift && grid3d_supported(latent_dim, feature_dim, grad_latents)) {
         if (zero_first) CUDA_OK(cudaMemsetAsync(grad_latents, 0, sizeof(float) * (size_t)table_rows * latent_dim, s));
         return backward_3d(const_cast<shacira_plan*>(plan), grad_output, nullptr, lp, latent_dim, feature_dim, A, per_level,
                            grad_latents, nullptr, nullptr, s);
@@ -555,10 +538,9 @@ int shacira_fit_tile_step(const shacira_plan_t* plan, const float* latents, cons
         CUDA_OK(cudaFuncSetAttribute(fit_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
     if (smem > 100 * 1024) return fail(SHACIRA_ERR_UNSUPPORTED, "fit_tile_step: %zu bytes of shared memory", smem);
     CUDA_OK(cudaMemsetAsync(mlp_out, 0, 8 + sizeof(float) * kFitParams, s));
-    static const int per_sm = [] { const char* e = getenv("SHACIRA_FIT_CTAS_PER_SM"); int v = e ? atoi(e) : 0; return v > 0 ? v : SHACIRA_FIT_MIN_CTAS; }();
-    int blocks = sm_count() * per_sm;
+    int blocks = sm_count() * SHACIRA_FIT_MIN_CTAS;
     if (blocks > p->ntiles) blocks = p->ntiles;
-    static const int headroom = [] { const char* e = getenv("SHACIRA_FIT_HEADROOM"); int v = e ? atoi(e) : 1; return v < 0 ? 0 : (v > 8 ? 8 : v); }();
+    const int headroom = 1;   // bits of slack of the fixed-point gradient scale (fit_kernels.cuh)
     const float scale = (float)(2.0 / ((double)p->n * 3.0));
     fit_tile_kernel<<<blocks, kTileThreads, smem, s>>>(view_of(p), latents, lp, A, shift, round_flag, target_sorted, W1, b1,
                                                        W2, b2, W3, b3, scale, grad_latents, grad_A, grad_shift,

@@ -685,7 +685,7 @@ latent_bwd_tiled_kernel(const PlanView pv, const float* __restrict__ grad_out, c
                         float* __restrict__ grad_shift, int cap, int cap_acc, const float* __restrict__ level_max,
                         int max_staged, int skip_direct) {
     // max_staged / skip_direct (3D): stage exactly the first max_staged levels (the host sized `cap` for them) and leave
-    // every other level to the point-parallel kernel that runs beside this one (latent_bwd3d_kernel, skip_mask).
+    // every other level to the lane-pair kernel that runs beside this one (latent_bwd3d_lp_kernel, skip_mask).
     constexpr bool SG = DEC && (F <= C);
     constexpr bool ZP = DEC && !SG;          // per-point z recomputation
     constexpr int CA = SG ? F : C;           // accumulator channels

@@ -103,7 +103,7 @@ class ImageFitStep:
         self.A = torch.empty((1, self.C, self.F), **f32)
         self.feats = torch.empty((self.n, self.L * self.F), **f32)
         self.gfeat = torch.empty_like(self.feats)
-        self.use_bound = self.IN == 16 and os.environ.get("SHACIRA_MLP_IMPL", "tc") == "tc"   # the tensor-core kernel
+        self.use_bound = self.IN == 16   # the tensor-core kernel
         # one tile-resident kernel for grid forward + MLP / MSE + grid backward where its shapes apply (SHACIRA_FIT_FUSED=0:
         # the three-kernel path, kept for every other shape and as the parity reference of the fused kernel)
         self.opt_fused = os.environ.get("SHACIRA_FIT_OPT_FUSED", "1") != "0"   # one optimizer launch (incl. next SGA sample)
