@@ -12,7 +12,6 @@ Prints one JSON line with the card's name and power limit read in the same run.
 """
 import argparse
 import json
-import math
 import os
 import subprocess
 import sys
@@ -26,7 +25,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "benchmarks"))
 import fit_image  # noqa: E402
 from shacira_b200 import _lib, grid_ops  # noqa: E402
-from shacira_b200.image_fit import ImageFitStep, _render, render_image  # noqa: E402
+from shacira_b200.image_fit import ImageFitStep, _render, lambda_at, render_image, temperature_at  # noqa: E402
 
 
 def card():
@@ -118,9 +117,9 @@ def recipe_round(dev, track, seeds, sga_steps, ste_steps, temperature=0.1, decay
 
     def host_side(k, it):
         fs = fits[k]
-        fs.set_lambda(1e-4 + 0.5 * (1e-3 - 1e-4) * (1 + math.cos(math.pi * it / total)))
+        fs.set_lambda(lambda_at(it, total))
         if fs.sga:
-            fs.set_temperature(fit_image.sga_temperature(it + 1, total, temperature, decay_period))
+            fs.set_temperature(temperature_at(it, total, temperature, decay_period))
         if it + 1 in (1, 2, 5, 10):
             fs.update_div()
 

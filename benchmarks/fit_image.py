@@ -33,6 +33,8 @@ import torch.nn as nn
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
+from shacira_b200.image_fit import lambda_at, temperature_at   # noqa: E402  the recipe's schedules
+
 H, W = 512, 768
 LATENT_SCALE = 20.0
 
@@ -111,12 +113,6 @@ def clamped_psnr(pred, gt):
     return 20 * np.log10(255.0) - 10 * np.log10(max(mse, 1e-12))
 
 
-def sga_temperature(epoch, num_epochs, end=0.1, decay_period=0.9):
-    """DecayScheduler('exp', start 1.0, end `temperature`) of the reference (utils/schedulers.py:21-23,
-    base_trainer.py:155-157): max(end, exp(-ln(1 / end) * epoch / num_epochs / decay_period))."""
-    return max(end, math.exp(-math.log(1.0 / end) * epoch / num_epochs / decay_period))
-
-
 def _native_setup(seed, dev, device_noise=False, sga=False):
     from shacira_b200.grids import LatentGrid
     from shacira_b200.image_fit import ImageFitStep
@@ -162,9 +158,9 @@ def fit_native_recipe(seeds, steps, dev, decay_period=0.9, temperature=0.1):
 
     def host_side(k, it):
         fs = fits[k][4]
-        fs.set_lambda(1e-4 + 0.5 * (1e-3 - 1e-4) * (1 + math.cos(math.pi * it / steps)))
+        fs.set_lambda(lambda_at(it, steps))
         if fs.sga:
-            fs.set_temperature(sga_temperature(it + 1, steps, temperature, decay_period))
+            fs.set_temperature(temperature_at(it, steps, temperature, decay_period))
         if it + 1 in (1, 2, 5, 10):
             fs.update_div()
 
@@ -223,7 +219,7 @@ def fit_native_many(seeds, steps, dev, use_graph, noise_cpu):
 
     def host_side(k, it):
         fs = fits[k][4]
-        fs.set_lambda(1e-4 + 0.5 * (1e-3 - 1e-4) * (1 + math.cos(math.pi * it / steps)))
+        fs.set_lambda(lambda_at(it, steps))
         if noise_cpu:
             fs.draw_noise(gens[k])      # otherwise the bit-rate kernel draws its own noise (device_noise)
         if it + 1 in (1, 2, 5, 10):
@@ -280,14 +276,14 @@ def fit_native_sga(seed, steps, dev, decay_period=0.9):
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     for it in range(steps):
-        fs.set_lambda(1e-4 + 0.5 * (1e-3 - 1e-4) * (1 + math.cos(math.pi * it / steps)))
+        fs.set_lambda(lambda_at(it, steps))
         fs.draw_noise(gen)
         if it + 1 in (1, 2, 5, 10):
             fs.update_div()
         on = it < int(decay_period * steps)
         if on != fs.sga:
             fs.set_sga(on)
-        fs.set_temperature(sga_temperature(it + 1, steps, 0.1, decay_period), refresh=True)
+        fs.set_temperature(temperature_at(it, steps, 0.1, decay_period), refresh=True)
         fs.sga_uniforms = torch.rand((T, 1, 2), generator=sga_gen).to(dev) if on else None
         fs.step()
     torch.cuda.synchronize()
@@ -370,7 +366,7 @@ def fit(seed, impl, steps, dev, use_graph, noise_cpu, fused_mlp=False, sga=False
 
     def host_side(it):
         # schedules and the noise draw happen outside the (possibly captured) device step
-        lam.fill_(1e-4 + 0.5 * (1e-3 - 1e-4) * (1 + math.cos(math.pi * it / steps)))   # schedulers.py:26-27
+        lam.fill_(lambda_at(it, steps))   # schedulers.py:26-27
         if noise_cpu:
             noise_buf.copy_(torch.rand((T, 1), generator=noise_gen) - 0.5)
         else:
@@ -382,7 +378,7 @@ def fit(seed, impl, steps, dev, use_graph, noise_cpu, fused_mlp=False, sga=False
         if sga:
             on = it < int(decay_period * steps)
             grid.latent_dec.use_sga = on
-            grid.latent_dec.temperature = sga_temperature(it + 1, steps, 0.1, decay_period)
+            grid.latent_dec.temperature = temperature_at(it, steps, 0.1, decay_period)
             grid.latent_dec.sga_uniforms = torch.rand((T, 1, 2), generator=sga_gen).to(dev) if on else None
 
     graph = None

@@ -503,6 +503,43 @@ int shacira_fit_optimizer_step_best(const shacira_adam_seg_t* segs, int32_t num_
                                     double* bits, float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes,
                                     uint32_t* ticket, const shacira_fit_snapshot_t* snap, shacira_stream_t stream);
 
+/* The trainer's schedules advanced by that launch (image_trainer.py:113-193; utils/schedulers.py). Before step `it`
+ * (0-based, = *step_small):
+ *   lambda(it) = lambda_end + 0.5 * (lambda_start - lambda_end) * (1 + cos(pi * it / num_epochs))   (COSINE)
+ *              = lambda_start                                                                      (FIX)
+ *   T(it)      = max(temperature_end, exp(-ln(1 / temperature_end) * (it + 1) / num_epochs / decay_period))
+ * evaluated in double and rounded to float. */
+#define SHACIRA_LAMBDA_FIX 0
+#define SHACIRA_LAMBDA_COSINE 1
+typedef struct {
+    int32_t num_epochs;          /* >= 1 */
+    int32_t lambda_kind;         /* SHACIRA_LAMBDA_COSINE or SHACIRA_LAMBDA_FIX */
+    double lambda_start, lambda_end;
+    double temperature_end;      /* > 0 */
+    double decay_period;         /* in (0, 1] */
+    const double* sse;           /* this step's rgb_loss = (float)(*sse / count), as for the snapshot */
+    int64_t count;
+    float* log;                  /* [log_capacity][4]: rgb_loss, total bits (NaN without bits), lambda, temperature */
+    int64_t log_capacity;
+} shacira_fit_schedule_t;
+/* shacira_fit_optimizer_step(_best) (snap may be NULL) that also advances the schedule: the last CTA appends record
+ * *step_small to sched->log (dropped when it is >= log_capacity) -- the step's rgb_loss, (float)bits[0] (the folded
+ * bit-rate loss of this launch, or what shacira_entropy_bits wrote before it), and the lambda (*scale2) and temperature
+ * (*temperature) the step used -- and then writes lambda(it + 1) into *scale2 and T(it + 1) into *temperature. Every
+ * reader of those scalars in the launch reads them first; the next step's SGA sample, drawn here, uses T(it). scale2
+ * and temperature must not be NULL. */
+int shacira_fit_optimizer_step_sched(const shacira_adam_seg_t* segs, int32_t num_segs, float* table, float* grad,
+                                     const float* grad_mul, const float* grad2, const float* scale2, float scale2_mul,
+                                     float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float weight_decay,
+                                     float beta1, float beta2, float eps, float* step_small, float* step_table,
+                                     const float* scale, const float* div, float* A_out, int32_t latent_dim,
+                                     int32_t feature_dim, const float* temperature, int32_t diff_sampling, uint64_t seed,
+                                     uint64_t* rng_step, float* w_hat, float* dw, const float* ent_params,
+                                     int32_t ent_layers, const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step,
+                                     double* bits, float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes,
+                                     uint32_t* ticket, const shacira_fit_snapshot_t* snap,
+                                     const shacira_fit_schedule_t* sched, shacira_stream_t stream);
+
 /* ---- exchange step of the ray-batch data-parallel path over NVLink / NVSwitch peer memory (SURVEY 8e) ------------
  * north_star: "NeRF ray batches are data-parallel, with the hash-table/latent gradient allreduced ... over NVLink".
  * The reference is single-GPU (no counterpart file); the NCCL form is shacira_b200.dp.GradArena.allreduce.

@@ -42,6 +42,17 @@ class FitSnapshot(ctypes.Structure):
     _fields_ = [("sse", _vp), ("count", _i64), ("best_loss", _vp), ("best_step", _vp), ("table", _vp),
                 ("seg_param", _vp * MAX_ADAM_SEGS), ("div", _vp), ("A", _vp)]
 
+
+LAMBDA_FIX = 0
+LAMBDA_COSINE = 1
+
+
+class FitSchedule(ctypes.Structure):
+    """shacira_fit_schedule_t (include/shacira_b200.h)."""
+    _fields_ = [("num_epochs", _i32), ("lambda_kind", _i32), ("lambda_start", ctypes.c_double),
+                ("lambda_end", ctypes.c_double), ("temperature_end", ctypes.c_double), ("decay_period", ctypes.c_double),
+                ("sse", _vp), ("count", _i64), ("log", _vp), ("log_capacity", _i64)]
+
 # name -> (restype, argtypes); mirrors include/shacira_b200.h one to one.
 SIGNATURES = {
     "shacira_abi_version": (ctypes.c_int, []),
@@ -88,6 +99,7 @@ SIGNATURES = {
     "shacira_peer_allreduce_adam": (ctypes.c_int, [ctypes.POINTER(_vp), _i64, _i32, _i32, _i64, ctypes.POINTER(_vp), _i64, _vp, _vp, _vp, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp]),
     "shacira_fit_optimizer_step": (ctypes.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _i32, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i32, _vp, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i64, _vp, _vp]),
     "shacira_fit_optimizer_step_best": (ctypes.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _i32, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i32, _vp, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp]),
+    "shacira_fit_optimizer_step_sched": (ctypes.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _i32, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i32, _vp, ctypes.c_uint64, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
     "shacira_adam_step": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _i32, _vp]),
     "shacira_adam_step_sum": (ctypes.c_int, [_vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _i32, _i32, _vp]),
     "shacira_adam_step_sum_mul": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, ctypes.c_float, _vp, _vp, _i64, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _i32, _i32, _vp]),

@@ -580,7 +580,8 @@ int fit_optimizer_launch(const shacira_adam_seg_t* segs, int32_t num_segs, float
                          float* w_hat, float* dw, const float* ent_params, int32_t ent_layers,
                          const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step, double* bits,
                          float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes, uint32_t* ticket,
-                         const shacira_fit_snapshot_t* snap, shacira_stream_t stream) {
+                         const shacira_fit_snapshot_t* snap, const shacira_fit_schedule_t* sched,
+                         shacira_stream_t stream) {
     if (!step_small || !step_table || !ticket || num_segs < 0 || (num_segs > 0 && !segs))
         return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step: NULL argument");
     if (num_segs > SHACIRA_MAX_ADAM_SEGS)
@@ -630,7 +631,16 @@ int fit_optimizer_launch(const shacira_adam_seg_t* segs, int32_t num_segs, float
         sn = *snap;
     }
     const int64_t blocks = num_segs + (n + 1023) / 1024;
-    if (snap)
+    if (sched) {
+        if (snap)
+            fit_optimizer_sched_kernel<true><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
+                S, Tb, beta1, beta2, eps, step_small, step_table, scale, div, A_out, latent_dim, feature_dim, ticket, sn,
+                *sched, bits);
+        else
+            fit_optimizer_sched_kernel<false><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
+                S, Tb, beta1, beta2, eps, step_small, step_table, scale, div, A_out, latent_dim, feature_dim, ticket, sn,
+                *sched, bits);
+    } else if (snap)
         fit_optimizer_kernel<true><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
             S, Tb, beta1, beta2, eps, step_small, step_table, scale, div, A_out, latent_dim, feature_dim, ticket, sn);
     else
@@ -658,7 +668,7 @@ int shacira_fit_optimizer_step(const shacira_adam_seg_t* segs, int32_t num_segs,
                                 lr, weight_decay, beta1, beta2, eps, step_small, step_table, scale, div, A_out,
                                 latent_dim, feature_dim, temperature, diff_sampling, seed, rng_step, w_hat, dw,
                                 ent_params, ent_layers, ent_noise, ent_seed, ent_rng_step, bits, grad_ent_params,
-                                ent_scratch, ent_scratch_bytes, ticket, nullptr, stream);
+                                ent_scratch, ent_scratch_bytes, ticket, nullptr, nullptr, stream);
 }
 
 int shacira_fit_optimizer_step_best(const shacira_adam_seg_t* segs, int32_t num_segs, float* table, float* grad,
@@ -676,7 +686,46 @@ int shacira_fit_optimizer_step_best(const shacira_adam_seg_t* segs, int32_t num_
                                 lr, weight_decay, beta1, beta2, eps, step_small, step_table, scale, div, A_out,
                                 latent_dim, feature_dim, temperature, diff_sampling, seed, rng_step, w_hat, dw,
                                 ent_params, ent_layers, ent_noise, ent_seed, ent_rng_step, bits, grad_ent_params,
-                                ent_scratch, ent_scratch_bytes, ticket, snap, stream);
+                                ent_scratch, ent_scratch_bytes, ticket, snap, nullptr, stream);
+}
+
+int shacira_fit_optimizer_step_sched(const shacira_adam_seg_t* segs, int32_t num_segs, float* table, float* grad,
+                                     const float* grad_mul, const float* grad2, const float* scale2, float scale2_mul,
+                                     float* exp_avg, float* exp_avg_sq, int64_t n, float lr, float weight_decay,
+                                     float beta1, float beta2, float eps, float* step_small, float* step_table,
+                                     const float* scale, const float* div, float* A_out, int32_t latent_dim,
+                                     int32_t feature_dim, const float* temperature, int32_t diff_sampling, uint64_t seed,
+                                     uint64_t* rng_step, float* w_hat, float* dw, const float* ent_params,
+                                     int32_t ent_layers, const float* ent_noise, uint64_t ent_seed, uint64_t* ent_rng_step,
+                                     double* bits, float* grad_ent_params, void* ent_scratch, int64_t ent_scratch_bytes,
+                                     uint32_t* ticket, const shacira_fit_snapshot_t* snap,
+                                     const shacira_fit_schedule_t* sched, shacira_stream_t stream) {
+    if (!sched) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: schedule descriptor is NULL");
+    if (!sched->log) return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: the step log is NULL");
+    if (sched->log_capacity < 0)
+        return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: log_capacity %lld < 0",
+                    (long long)sched->log_capacity);
+    if (!sched->sse || sched->count <= 0)
+        return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: sse / count missing");
+    if (sched->num_epochs < 1)
+        return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: num_epochs %d < 1", sched->num_epochs);
+    if (!(sched->decay_period > 0.0 && sched->decay_period <= 1.0))
+        return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: decay_period %g outside (0, 1]",
+                    sched->decay_period);
+    if (!(sched->temperature_end > 0.0))
+        return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: temperature_end %g <= 0",
+                    sched->temperature_end);
+    if (sched->lambda_kind != SHACIRA_LAMBDA_COSINE && sched->lambda_kind != SHACIRA_LAMBDA_FIX)
+        return fail(SHACIRA_ERR_UNSUPPORTED, "fit_optimizer_step_sched: unknown lambda kind %d", sched->lambda_kind);
+    if (!scale2 || !temperature)
+        return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: the lambda (scale2) and temperature scalars are NULL");
+    if (reinterpret_cast<uintptr_t>(sched->log) & 15)
+        return fail(SHACIRA_ERR_INVALID_ARGUMENT, "fit_optimizer_step_sched: the step log must be 16-byte aligned");
+    return fit_optimizer_launch(segs, num_segs, table, grad, grad_mul, grad2, scale2, scale2_mul, exp_avg, exp_avg_sq, n,
+                                lr, weight_decay, beta1, beta2, eps, step_small, step_table, scale, div, A_out,
+                                latent_dim, feature_dim, temperature, diff_sampling, seed, rng_step, w_hat, dw,
+                                ent_params, ent_layers, ent_noise, ent_seed, ent_rng_step, bits, grad_ent_params,
+                                ent_scratch, ent_scratch_bytes, ticket, snap, sched, stream);
 }
 
 int shacira_multi_adam_step(const shacira_adam_seg_t* segs, int32_t num_segs, float beta1, float beta2, float eps,

@@ -27,18 +27,96 @@ The module parameters stay the single source of truth: the kernels read and upda
 `grid.codebook`, `grid.latent_dec.layers[0].{scale,shift}`, `grid.prob_model.f*.{h,b,a}` and the MLP in place, so
 `grid.interpolate`, `grid.size()`, `state_dict()` etc. see the trained values at any time.
 
+The trainer's schedules can run on the device too (image_trainer.py:113-193): after `set_schedule(recipe)` the optimizer
+launch writes the next step's lambda and SGA temperature itself and appends every step's rgb_loss / bits / lambda /
+temperature to a device log (`history`), so a CUDA graph of K captured steps is K schedule steps with no host work.
+`fit_image` / `fit_images` run the reference's whole recipe (`ImageRecipe`, kodak.yaml) that way.
+
 Model selection and evaluation stay on the device as well (image_trainer.py:173-178,305-310,471-502): with
 track_best=True the optimizer launch keeps the parameters of the lowest rgb_loss seen so far (`best_loss`, `best_step`,
 `restore_best`), and `render` / `render_image` turn a model of the fused kernel's shape into pixels and its clamped
 PSNR in one forward-only kernel (shacira_fit_render).
 """
 import ctypes
+import dataclasses
 import math
 import os
 
 import torch
 
 from . import _lib, grid_ops
+
+_LAMBDA_KINDS = {"cosine": _lib.LAMBDA_COSINE, "fix": _lib.LAMBDA_FIX}
+
+
+def lambda_at(it, num_epochs, start=1e-3, end=1e-4, kind="cosine"):
+    """Bit-rate weight lambda before step `it` (0-based) of a `num_epochs` fit (utils/schedulers.py, 'cosine' or 'fix').
+    The optimizer launch of a scheduled ImageFitStep evaluates the same expression on the device."""
+    if kind == "fix":
+        return start
+    if kind != "cosine":
+        raise _lib.ShaciraError(_lib.ERR_UNSUPPORTED, "unknown lambda schedule %r" % (kind,))
+    return end + 0.5 * (start - end) * (1 + math.cos(math.pi * it / num_epochs))
+
+
+def temperature_at(it, num_epochs, end=0.1, decay_period=0.9):
+    """SGA temperature before step `it` (0-based): the reference's DecayScheduler('exp', start 1.0, end) at epoch it + 1
+    (utils/schedulers.py:21-23, base_trainer.py:155-157)."""
+    return max(end, math.exp(-math.log(1.0 / end) * (it + 1) / num_epochs / decay_period))
+
+
+@dataclasses.dataclass(frozen=True)
+class ImageRecipe:
+    """The reference's Kodak training recipe (app/image/configs/kodak.yaml; Adam groups of base_trainer.py:219-239):
+    `epochs` full-image steps; lambda from `lambda_start` to `lambda_end` ('cosine') or fixed at `lambda_start` ('fix');
+    SGA with temperature 1 -> `temperature_end` while epoch / epochs <= `decay_period`, straight-through rounding after;
+    norm='max' div updates before the steps of `div_epochs` (1-based); bit-rate noise drawn on the device."""
+    epochs: int = 60_000
+    lr: float = 1e-3
+    grid_lr: float = 2e-2
+    ldec_lr: float = 1e-2
+    prob_lr: float = 1e-4
+    weight_decay: float = 0.0
+    weight_decay_decoder: float = 1e-2
+    betas: tuple = (0.9, 0.999)
+    eps: float = 1e-8
+    lambda_start: float = 1e-3
+    lambda_end: float = 1e-4
+    lambda_kind: str = "cosine"
+    temperature_end: float = 0.1
+    decay_period: float = 0.9
+    div_epochs: tuple = (1, 2, 5, 10)
+    device_noise: bool = True
+
+    def __post_init__(self):
+        bad = lambda msg: _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "ImageRecipe: " + msg)
+        if int(self.epochs) < 1 or (self.div_epochs and int(self.epochs) < max(self.div_epochs)):
+            raise bad("epochs %r: at least 1 and at least the last div epoch %r" % (self.epochs, self.div_epochs))
+        if any(int(e) < 1 for e in self.div_epochs):
+            raise bad("div epochs count from 1")
+        if not 0.0 < float(self.decay_period) <= 1.0:
+            raise bad("decay_period %r outside (0, 1]" % (self.decay_period,))
+        if not float(self.temperature_end) > 0.0:
+            raise bad("temperature_end %r must be > 0" % (self.temperature_end,))
+        if self.lambda_kind not in _LAMBDA_KINDS:
+            raise _lib.ShaciraError(_lib.ERR_UNSUPPORTED, "ImageRecipe: unknown lambda kind %r" % (self.lambda_kind,))
+
+    @property
+    def switch(self):
+        """The first straight-through step: SGA while epoch / epochs <= decay_period (image_trainer.py:136-137)."""
+        return int(math.floor(self.decay_period * self.epochs))
+
+    def lambda_at(self, it):
+        return lambda_at(it, self.epochs, self.lambda_start, self.lambda_end, self.lambda_kind)
+
+    def temperature_at(self, it):
+        return temperature_at(it, self.epochs, self.temperature_end, self.decay_period)
+
+    def step_kwargs(self):
+        """The ImageFitStep arguments of this recipe."""
+        return dict(lr=self.lr, grid_lr=self.grid_lr, ldec_lr=self.ldec_lr, prob_lr=self.prob_lr,
+                    weight_decay=self.weight_decay, weight_decay_decoder=self.weight_decay_decoder, betas=self.betas,
+                    eps=self.eps, device_noise=self.device_noise)
 
 
 class ImageFitStep:
@@ -222,6 +300,44 @@ class ImageFitStep:
                 snap.seg_param[i] = b.data_ptr()
             self.snap = snap
         self.sse_u8 = torch.zeros((), dtype=torch.int64, device=dev)
+        self.sched = None
+
+    # ---- device-side schedule ---------------------------------------------------------------------
+    def set_schedule(self, recipe, log_capacity=None):
+        """From the next step on, the optimizer launch advances lambda and the SGA temperature itself (the values of
+        recipe.lambda_at / recipe.temperature_at at the step counter) and logs every step (`history`) at its index, for
+        the first `log_capacity` steps (default recipe.epochs). set_lambda / set_temperature still overwrite the device
+        scalars; the launch replaces them after the next step. Needs the one-launch optimizer. A CUDA graph captured
+        before this call keeps the previous schedule and log (kept alive here): re-capture after calling it."""
+        if not self.opt_fused:
+            raise _lib.ShaciraError(_lib.ERR_UNSUPPORTED, "ImageFitStep: a device-side schedule needs the one-launch "
+                                                          "optimizer (SHACIRA_FIT_OPT_FUSED=0 is set)")
+        cap = int(recipe.epochs if log_capacity is None else log_capacity)
+        if cap < 0:
+            raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "ImageFitStep.set_schedule: log_capacity < 0")
+        if self.sched is not None:
+            self._keep.append(self.log)   # a graph captured earlier still writes into the previous log
+        self.log = torch.full((max(cap, 1), 4), float("nan"), dtype=torch.float32, device=self.dev)
+        sc = _lib.FitSchedule()
+        sc.num_epochs, sc.lambda_kind = int(recipe.epochs), _LAMBDA_KINDS[recipe.lambda_kind]
+        sc.lambda_start, sc.lambda_end = float(recipe.lambda_start), float(recipe.lambda_end)
+        sc.temperature_end, sc.decay_period = float(recipe.temperature_end), float(recipe.decay_period)
+        sc.sse, sc.count = self.mlp_out.data_ptr(), self.n * self.OUT
+        sc.log, sc.log_capacity = self.log.data_ptr(), cap
+        self.sched, self.recipe = sc, recipe
+        it = int(self.step_small)
+        self.set_lambda(recipe.lambda_at(it))
+        self.set_temperature(recipe.temperature_at(it))
+
+    def history(self):
+        """The step log of the scheduled steps as float32 device tensors, one entry per step taken (up to the log's
+        capacity): rgb_loss (bit for bit rgb_loss()), bits (total_bits()), and the lambda and temperature the step used.
+        Reads the step counter on the host."""
+        if self.sched is None:
+            raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "ImageFitStep.history: no schedule (set_schedule)")
+        k = min(int(self.step_small), int(self.sched.log_capacity))
+        log = self.log[:k]
+        return dict(rgb_loss=log[:, 0], bits=log[:, 1], lam=log[:, 2], temperature=log[:, 3])
 
     # ---- host-side schedule hooks ------------------------------------------------------------
     def refresh_A(self):
@@ -354,7 +470,10 @@ class ImageFitStep:
                     None if self.device_noise else P(self.noise), self.noise_seed,
                     P(self.rng_step), P(self.bits), P(self.g_prob), P(self.ent_scratch),
                     self.ent_scratch.numel(), P(self.adam_ticket)]
-            if self.track_best:   # the same launch, snapshotting the parameters of an improving step
+            if self.sched is not None:   # the same launch, advancing lambda / temperature and logging the step
+                chk(lib.shacira_fit_optimizer_step_sched(*args, ctypes.byref(self.snap) if self.track_best else None,
+                                                         ctypes.byref(self.sched), st))
+            elif self.track_best:   # the same launch, snapshotting the parameters of an improving step
                 chk(lib.shacira_fit_optimizer_step_best(*args, ctypes.byref(self.snap), st))
             else:
                 chk(lib.shacira_fit_optimizer_step(*args, st))
@@ -440,20 +559,26 @@ def _psnr(sse, count):
     return 20.0 * math.log10(255.0) - 10.0 * torch.log10(mse)
 
 
+def _renders(grid, mlp):
+    """True for a model of the fused fit kernel's shape (what render_image / shacira_fit_render take)."""
+    dec = grid.latent_dec
+    amap = dec.affine_map() if hasattr(dec, "affine_map") else None
+    lin = [mlp[0], mlp[2], mlp[4]] if len(mlp) == 5 else None
+    return not (amap is None or amap[0].shape[0] != 1 or "dft" in getattr(dec.layers[0], "ldecode_matrix", "") or
+                grid.resolution_dim != 2 or grid.num_lods != 16 or tuple(grid.codebook.shape[1:]) != (1,) or
+                tuple(amap[0].shape) != (1, 1, 1) or lin is None or
+                [(l.in_features, l.out_features) for l in lin] != [(16, 16), (16, 16), (16, 3)])
+
+
 def render_image(grid, mlp, coords, target=None):
     """mlp(grid.interpolate(coords)) for a model of the fused fit kernel's shape -- 2D LatentGrid with 16 levels,
     latent_dim = feature_dim = 1, one affine 'sq' latent decoder, MLP 16 -> 16 -> 16 -> 3 -- in one forward-only kernel
     with the latents rounded: a trained or a decoded codec model, on any coordinate set (e.g. a 2x upsampled pixel
     grid). Returns (rgb [N, 3] in the order of `coords`, clamped PSNR against `target` [N, 3] as a float64 device
     scalar, or None without a target). Other shapes raise ShaciraError (use mlp(grid.interpolate(coords)))."""
-    dec = grid.latent_dec
-    amap = dec.affine_map() if hasattr(dec, "affine_map") else None
-    lin = [mlp[0], mlp[2], mlp[4]] if len(mlp) == 5 else None
-    if (amap is None or amap[0].shape[0] != 1 or "dft" in getattr(dec.layers[0], "ldecode_matrix", "") or
-            grid.resolution_dim != 2 or grid.num_lods != 16 or tuple(grid.codebook.shape[1:]) != (1,) or
-            tuple(amap[0].shape) != (1, 1, 1) or lin is None or
-            [(l.in_features, l.out_features) for l in lin] != [(16, 16), (16, 16), (16, 3)]):
+    if not _renders(grid, mlp):
         raise _lib.ShaciraError(_lib.ERR_UNSUPPORTED, "render_image: needs the fused fit kernel's model shape")
+    lin = [mlp[0], mlp[2], mlp[4]]
     coords = _lib._f32c(coords, "coords")
     n = coords.shape[0]
     if coords.dim() != 2 or coords.shape[1] != 2:
@@ -469,7 +594,7 @@ def render_image(grid, mlp, coords, target=None):
         plan = _lib.Plan(coords, tile_points=32)
     fi, _ = _lib._i32_array(grid._first_idx())
     rs, L = _lib._i32_array(grid.resolutions)
-    A, shift = amap
+    A, shift = grid.latent_dec.affine_map()
     with torch.no_grad():
         A = A.detach().contiguous()
         shift = shift.detach().contiguous() if shift is not None else None
@@ -479,3 +604,136 @@ def render_image(grid, mlp, coords, target=None):
         _render(plan, _lib._f32c(grid.codebook.data, "codebook"), fi, rs, L, int(grid.codebook_bitwidth), A, shift, lin,
                 rgb, target, sse)
     return rgb, (_psnr(sse, n * 3) if target is not None else None)
+
+
+def _clamped_psnr(pred, target):
+    """clamped_psnr (wisp/ops/image/metrics.py:39-57) of a prediction against its target: float64 device scalar."""
+    q = lambda v: (torch.clamp(v, 0, 1) * 255).to(torch.uint8).to(torch.int64)
+    return _psnr(((q(pred) - q(target)) ** 2).sum(), pred.numel())
+
+
+def fit_image(grid, mlp, coords, target, recipe=ImageRecipe(), chunk=100, noise_seed=0):
+    """Fit one image with the reference's training recipe (ImageTrainer, image_trainer.py:113-193,269-359,471-514):
+    fit_images with one fit in flight. Returns its result dict (see fit_images)."""
+    return fit_images([(grid, mlp, coords, target)], recipe, in_flight=1, chunk=chunk, noise_seeds=[noise_seed])[0]
+
+
+def fit_images(fits, recipe=ImageRecipe(), in_flight=3, chunk=100, noise_seeds=None):
+    """Independent fits [(grid, mlp, coords, target), ...] with `recipe`, `in_flight` at a time on one stream and one set
+    of CUDA graphs each (independent fits overlap each other's latency). Every model ImageFitStep takes is accepted.
+
+    Each fit runs an ImageFitStep with track_best and the recipe's device-side schedule: the first max(div_epochs) steps
+    (at least one) eagerly, with update_div before the steps of div_epochs; then the SGA phase and, from step floor(decay_period x
+    epochs), the straight-through phase, each as replays of one captured graph of `chunk` steps plus one of the
+    remainder. The best state is restored into the modules at the end.
+
+    Returns one dict per fit: best_step, best_loss (lowest rgb_loss and its 0-based step), psnr (clamped PSNR of the best
+    state: render_image where the model has the fused shape, mlp(grid.interpolate(coords)) otherwise), blob
+    (codec.encode_model), size (codec.size_report: reference-formula and file bpp), history (ImageFitStep.history,
+    device tensors), steps and device_ms per phase ('eager', 'sga', 'ste': CUDA-event time on the fit's stream)."""
+    from . import codec
+    if int(chunk) < 1:
+        raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "fit_images: chunk %r < 1" % (chunk,))
+    if int(in_flight) < 1:
+        raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "fit_images: in_flight %r < 1" % (in_flight,))
+    fits = list(fits)
+    seeds = list(noise_seeds) if noise_seeds is not None else list(range(len(fits)))
+    if len(seeds) != len(fits):
+        raise _lib.ShaciraError(_lib.ERR_INVALID_ARGUMENT, "fit_images: one noise seed per fit")
+    out = []
+    for g0 in range(0, len(fits), int(in_flight)):
+        runs = []
+        try:
+            for f, s in zip(fits[g0:g0 + int(in_flight)], seeds[g0:g0 + int(in_flight)]):
+                runs.append(_RecipeFit(*f, recipe, s))
+            _run_recipe(runs, recipe, int(chunk))
+            out += [r.result(codec) for r in runs]
+        finally:
+            for r in runs:
+                r.fs.close()
+    return out
+
+
+class _RecipeFit:
+    """One fit of fit_images: its ImageFitStep, stream, and per-phase events."""
+
+    def __init__(self, grid, mlp, coords, target, recipe, noise_seed):
+        self.grid, self.mlp, self.coords, self.target = grid, mlp, coords, target
+        self.fs = ImageFitStep(grid, mlp, coords, target, noise_seed=noise_seed, track_best=True, **recipe.step_kwargs())
+        self.fs.set_sga(recipe.switch > 0)
+        self.fs.set_schedule(recipe)
+        self.stream = torch.cuda.Stream(device=self.fs.dev)
+        self.events = {}
+        self.steps = {}
+
+    def mark(self, phase, end):
+        ev = torch.cuda.Event(enable_timing=True)
+        ev.record(self.stream)
+        self.events.setdefault(phase, [None, None])[1 if end else 0] = ev
+
+    def capture(self, k):
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g, stream=self.stream):
+            for _ in range(k):
+                self.fs.step()
+        return g
+
+    def result(self, codec):
+        fs = self.fs
+        if fs.sga:
+            fs.set_sga(False)   # evaluate the rounded model (decay_period = 1 never reaches the STE phase)
+        fs.restore_best()
+        with torch.no_grad():
+            if _renders(self.grid, self.mlp):
+                psnr = render_image(self.grid, self.mlp, self.coords, self.target)[1]
+            else:
+                psnr = _clamped_psnr(self.mlp(self.grid.interpolate(self.coords, 0)), self.target)
+        blob = codec.encode_model(self.grid, self.mlp)
+        return dict(best_step=int(fs.best_step()), best_loss=float(fs.best_loss()), psnr=float(psnr), blob=blob,
+                    size=codec.size_report(self.grid, self.mlp, blob, self.coords.shape[0]),
+                    history={k: v.clone() for k, v in fs.history().items()}, steps=dict(self.steps),
+                    device_ms={p: e[0].elapsed_time(e[1]) for p, e in self.events.items()})
+
+
+def _run_recipe(runs, recipe, chunk):
+    epochs, switch = recipe.epochs, recipe.switch
+    # at least one eager step: it draws the first SGA sample, so that every captured step takes the one the previous
+    # optimizer launch drew (as the host-driven loop does) instead of redrawing it
+    eager = max(1, min(max(recipe.div_epochs, default=0), epochs))
+    torch.cuda.synchronize()
+    for r in runs:
+        r.mark("eager", False)
+    for it in range(eager):
+        for r in runs:
+            with torch.cuda.stream(r.stream):
+                if it == switch:
+                    r.fs.set_sga(False)
+                if it + 1 in recipe.div_epochs:
+                    r.fs.update_div()
+                r.fs.step()
+    for r in runs:
+        r.mark("eager", True)
+        r.steps["eager"] = eager
+    for phase, a, b in (("sga", eager, switch), ("ste", max(eager, switch), epochs)):
+        if b <= a:
+            continue
+        full, rem = divmod(b - a, chunk)
+        for r in runs:
+            if phase == "ste" and r.fs.sga:
+                r.fs.set_sga(False)   # a captured graph holds its quantiser
+        # capture synchronises the device; it records the steps without running them
+        graphs = [(r.capture(chunk) if full else None, r.capture(rem) if rem else None) for r in runs]
+        for r in runs:
+            r.mark(phase, False)
+        for _ in range(full):
+            for r, (g, _g) in zip(runs, graphs):
+                with torch.cuda.stream(r.stream):
+                    g.replay()
+        for r, (_g, g) in zip(runs, graphs):
+            if g is not None:
+                with torch.cuda.stream(r.stream):
+                    g.replay()
+        for r in runs:
+            r.mark(phase, True)
+            r.steps[phase] = b - a
+    torch.cuda.synchronize()
