@@ -273,6 +273,10 @@ class PeerTable:
         self.m_base = self.m.data_ptr() - 4 * begin
         self.v_base = self.v.data_ptr() - 4 * begin
         self.step = torch.zeros((), dtype=torch.float32, device=dev)
+        # allreduce_adam() advances `step` right behind this rank's exchange kernel. The first launch of that add can
+        # load its kernel, and loading can wait for the device to go idle: in a process that launches several ranks,
+        # that would wait on an exchange that waits for the next rank's launch until the barriers give up. Load it here.
+        self.step += 0.0
         self.slice = (begin, end)
 
     def close(self):
