@@ -111,8 +111,15 @@ int launch_fwd(shacira_plan* p, const float* lat, const LevelParams& lp, const f
     const size_t rows_bytes = ((smem + 15) & ~(size_t)15) - smem + sizeof(float) * (size_t)kTileThreads * kPts * (RL + 4 + 1);
     const int rows_via_smem = !p->sorted_io && RL % 4 == 0 && RL <= 64 && smem + rows_bytes <= 46 * 1024;
     if (rows_via_smem) smem += rows_bytes;
-    latent_fwd_tiled_kernel<D, C, F><<<p->ntiles, kTileThreads, smem, s>>>(view_of(p), lat, lp, A, shift, per_level,
-                                                                            round_flag, feats, cap, rows_via_smem);
+    // 2D: the next batch's permutation entries and coordinates in slots behind the rows (or the decoder), unless they
+    // would take the launch past 46 KB (48 KB with the static part); that launch loads them directly
+    const size_t smem_pts = ((smem + 15) & ~(size_t)15) + kFwdPointSlotBytes;
+    if (D == 2 && smem_pts <= 46 * 1024)
+        latent_fwd_tiled_kernel<D, C, F, D == 2><<<p->ntiles, kTileThreads, smem_pts, s>>>(
+            view_of(p), lat, lp, A, shift, per_level, round_flag, feats, cap, rows_via_smem);
+    else
+        latent_fwd_tiled_kernel<D, C, F, false><<<p->ntiles, kTileThreads, smem, s>>>(view_of(p), lat, lp, A, shift, per_level,
+                                                                                   round_flag, feats, cap, rows_via_smem);
     LAUNCHED();
     return SHACIRA_OK;
 }
@@ -136,11 +143,26 @@ int launch_bwd(shacira_plan* p, const float* g, const float* lat, const LevelPar
     constexpr int NW = kTileThreads / 32;
     size_t smem = sizeof(float) * ((size_t)cap_acc * CA + (dec ? (size_t)cap * C : 0) + nA * C * F);
     if (dec) smem += sizeof(float) * (size_t)(zp ? NW : 1) * lp.num_lods * (C * F + F);
+    // 2D: the next-chunk slots, unless they would take the launch past 46 KB (48 KB with the static part) -- the
+    // largest node boxes, which keep the register loop
+    const size_t smem_pipe = ((smem + 15) & ~(size_t)15) + bwd_slot_bytes(D, F);
+    if constexpr (bwd_pipelined(D, F)) {
+        if (smem_pipe <= 46 * 1024) {
+            if (dec)
+                latent_bwd_tiled_kernel<D, C, F, true, true><<<p->ntiles, kTileThreads, smem_pipe, s>>>(
+                    view_of(p), g, lat, lp, A, per_level, round_flag, gl, gA, gS, cap, cap_acc, level_max, SHACIRA_MAX_LEVELS, 0);
+            else
+                latent_bwd_tiled_kernel<D, C, F, false, true><<<p->ntiles, kTileThreads, smem_pipe, s>>>(
+                    view_of(p), g, lat, lp, A, per_level, round_flag, gl, gA, gS, cap, cap_acc, level_max, SHACIRA_MAX_LEVELS, 0);
+            LAUNCHED();
+            return SHACIRA_OK;
+        }
+    }
     if (dec)
-        latent_bwd_tiled_kernel<D, C, F, true><<<p->ntiles, kTileThreads, smem, s>>>(view_of(p), g, lat, lp, A, per_level,
+        latent_bwd_tiled_kernel<D, C, F, true, false><<<p->ntiles, kTileThreads, smem, s>>>(view_of(p), g, lat, lp, A, per_level,
                                                                                       round_flag, gl, gA, gS, cap, cap_acc, level_max, SHACIRA_MAX_LEVELS, 0);
     else
-        latent_bwd_tiled_kernel<D, C, F, false><<<p->ntiles, kTileThreads, smem, s>>>(view_of(p), g, lat, lp, A, per_level,
+        latent_bwd_tiled_kernel<D, C, F, false, false><<<p->ntiles, kTileThreads, smem, s>>>(view_of(p), g, lat, lp, A, per_level,
                                                                                        round_flag, gl, gA, gS, cap, cap_acc, level_max, SHACIRA_MAX_LEVELS, 0);
     LAUNCHED();
     return SHACIRA_OK;

@@ -19,6 +19,8 @@
 // Indices, weights and rounding are computed by the same device functions as the point-parallel
 // kernels (common.cuh), so hash indices and quantised latents stay bit-identical to the reference.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace shacira {
@@ -449,10 +451,34 @@ constexpr int kStageUnroll = SHACIRA_STAGE_UNROLL;
 #ifndef SHACIRA_LV
 #define SHACIRA_LV 4
 #endif
-#ifndef SHACIRA_BWD_PREFETCH
-#define SHACIRA_BWD_PREFETCH 0   // measured: the extra row registers spill at the 72-register cap (38.1 vs 36.7 us)
-#endif
 constexpr int kLv = SHACIRA_LV;  // levels per inner iteration (register blocking of the level loop): 4 or 2
+
+// Asynchronous global -> shared copies (LDGSTS): the data goes to a thread-private shared-memory slot without
+// holding registers while it is in flight. src_bytes = 0 fills the slot with zeros and reads nothing.
+__device__ __forceinline__ void cp_async16(void* dst, const void* src, int src_bytes) {
+    asm volatile("cp.async.cg.shared.global.L2::64B [%0], [%1], 16, %2;\n"
+                 :: "r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src), "r"(src_bytes) : "memory");
+}
+template <int N>   // 4 or 8 bytes
+__device__ __forceinline__ void cp_async_small(void* dst, const void* src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], %2;\n"
+                 :: "r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src), "n"(N) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;\n" ::: "memory"); }
+
+// Points per thread of one register batch of the backward, and whether the 2D backward can request the next level
+// chunk's gradient pieces into shared-memory slots ([KB][kLv * F / 4][kTileThreads] float4 at the end of the
+// dynamic shared memory, bwd_slot_bytes) while the current chunk is reduced and accumulated. F = 8 (16 KB of slots)
+// keeps the register loop, and so does a launch whose node boxes leave no room for the slots (launch_bwd).
+__host__ __device__ constexpr int bwd_points_per_thread(int F) { return (F == 1) ? 3 : ((F == 2) ? 2 : 1); }
+__host__ __device__ constexpr bool bwd_pipelined(int D, int F) { return D == 2 && F <= 4; }
+__host__ __device__ constexpr int bwd_slot_bytes(int D, int F) {
+    return bwd_pipelined(D, F) ? bwd_points_per_thread(F) * kLv * F * 4 * kTileThreads : 0;
+}
+// 2D forward: permutation entries and coordinates of one batch of kPts points per thread, requested into
+// shared-memory slots one batch ahead (int [kPts][kTileThreads], then float2 [kPts][kTileThreads]).
+constexpr int kFwdPointSlotBytes = kPts * kTileThreads * (4 + 8);
 template <int D, int C>
 __device__ __forceinline__ void stage_nodes(const TileGeom<D>& tg, const int2* __restrict__ tab,
                                             const float* __restrict__ latents, int round_flag, float* s_nodes) {
@@ -539,7 +565,9 @@ plan_nodes_kernel(const __grid_constant__ LevelParams lp, int g, int cap, int2* 
 // ---------------------------------------------------------------------------------------------
 // forward: 4 levels per iteration, outputs written as 16-byte vectors (needs num_lods % 4 == 0)
 // ---------------------------------------------------------------------------------------------
-template <int D, int C, int F>
+// PTS (2D, when the slots fit beside the node box): a batch's permutation entries and coordinates arrive through
+// shared-memory slots one batch ahead (kFwdPointSlotBytes; launch_fwd decides).
+template <int D, int C, int F, bool PTS>
 __global__ void __launch_bounds__(kTileThreads, (C * F <= 4) ? SHACIRA_MIN_CTAS : 3)
 latent_fwd_tiled_kernel(const PlanView pv, const float* __restrict__ latents, const __grid_constant__ LevelParams lp,
                         const float* __restrict__ A, const float* __restrict__ shift, int per_level, int round_flag,
@@ -566,6 +594,24 @@ latent_fwd_tiled_kernel(const PlanView pv, const float* __restrict__ latents, co
 #pragma unroll
         for (int d = 0; d < D; ++d) { ti[d] = r % pv.g; r /= pv.g; }
     }
+    static_assert(!PTS || D == 2, "the point slots hold 2D coordinates");
+    // the point slots follow the row buffer, or the decoder when there is none
+    char* s_pts = reinterpret_cast<char*>(s_rows) + (rows_via_smem ? sizeof(float) * kTileThreads * kPts * (RS + 1) : 0);
+    int* s_pperm = reinterpret_cast<int*>(s_pts);
+    float2* s_pxy = reinterpret_cast<float2*>(s_pts + sizeof(int) * kTileThreads * kPts);
+    // requests this thread's permutation entries and coordinates of the batch at `base` into its own slots
+    auto request_points = [&](int base) {
+#pragma unroll
+        for (int k = 0; k < kPts; ++k) {
+            const int j = base + k * kTileThreads + threadIdx.x;
+            if (j < end) {
+                if (pv.perm) cp_async_small<4>(s_pperm + k * kTileThreads + threadIdx.x, pv.perm + j);
+                cp_async_small<8>(s_pxy + k * kTileThreads + threadIdx.x, pv.coords_sorted + (int64_t)j * 2);
+            }
+        }
+        cp_async_commit();
+    };
+    if constexpr (PTS) request_points(beg);   // in flight during the staging below
     const int2* tab = pv.node_tab + (size_t)tile * pv.node_stride;
     int pre[kPre];
     prefetch_rows(tab, pv.node_stride, pre);
@@ -579,15 +625,33 @@ latent_fwd_tiled_kernel(const PlanView pv, const float* __restrict__ latents, co
         // kPts points per thread: permutation entries and coordinates of all of them are requested first
         int orig[kPts];
         double t[kPts][D];
+        if constexpr (PTS) {
+            // this batch's points arrived in the thread's slots; the next batch's are requested behind this one
+            cp_async_wait_all();
 #pragma unroll
-        for (int k = 0; k < kPts; ++k) {
-            const int j = base + k * kTileThreads + threadIdx.x;
-            orig[k] = -1;
+            for (int k = 0; k < kPts; ++k) {
+                const int j = base + k * kTileThreads + threadIdx.x;
+                orig[k] = -1;
+                t[k][0] = t[k][1] = 0.5;
+                if (j < end) {
+                    orig[k] = pv.perm ? s_pperm[k * kTileThreads + threadIdx.x] : j;
+                    const float2 c = s_pxy[k * kTileThreads + threadIdx.x];
+                    t[k][0] = unit_coord(c.x);
+                    t[k][1] = unit_coord(c.y);
+                }
+            }
+            if (base + kTileThreads * kPts < end) request_points(base + kTileThreads * kPts);
+        } else {
 #pragma unroll
-            for (int d = 0; d < D; ++d) t[k][d] = 0.5;
-            if (j < end) {
-                orig[k] = pv.perm ? __ldg(pv.perm + j) : j;
-                load_unit_coords<D>(pv.coords_sorted, j, t[k]);
+            for (int k = 0; k < kPts; ++k) {
+                const int j = base + k * kTileThreads + threadIdx.x;
+                orig[k] = -1;
+#pragma unroll
+                for (int d = 0; d < D; ++d) t[k][d] = 0.5;
+                if (j < end) {
+                    orig[k] = pv.perm ? __ldg(pv.perm + j) : j;
+                    load_unit_coords<D>(pv.coords_sorted, j, t[k]);
+                }
             }
         }
         for (int l0 = 0; l0 < L; l0 += kLv) {
@@ -677,7 +741,7 @@ __device__ __forceinline__ int fixed_rn(float v) { return __float_as_int(__fadd_
 //       per node (F channels). Everything else is linear in G and is applied ONCE PER NODE at flush time:
 //       grad_latent[node] = A G[node];  grad_A += q[node] G[node]^T;  grad_shift += G[node]  (sum_k w_k = 1).
 //       That is ~2-3 nodes per point instead of 2^D * L corner visits per point.
-template <int D, int C, int F, bool DEC>
+template <int D, int C, int F, bool DEC, bool PIPE = bwd_pipelined(D, F)>
 __global__ void __launch_bounds__(kTileThreads, (C * F <= 4) ? SHACIRA_MIN_CTAS : 3)
 latent_bwd_tiled_kernel(const PlanView pv, const float* __restrict__ grad_out, const float* __restrict__ latents,
                         const __grid_constant__ LevelParams lp, const float* __restrict__ A, int per_level,
@@ -713,6 +777,93 @@ latent_bwd_tiled_kernel(const PlanView pv, const float* __restrict__ grad_out, c
 #pragma unroll
         for (int d = 0; d < D; ++d) { ti[d] = r % pv.g; r /= pv.g; }
     }
+
+    // Points per thread held in registers for a whole batch: each 16-byte piece of a gradient row is read ONCE, its
+    // levels' maxima (the fixed-point scales) are reduced from the registers, and after one barrier the same registers
+    // feed the accumulation -- no separate max pass over the rows (round 1: a second, latency-bound read of every row).
+    // A tile with more points than one register batch (uneven sample sets; the test suite's clustered case) runs the
+    // max pass of round 1 over up to kBatch points first and then several register batches into the SAME accumulators:
+    // one zero-fill and one flush per kBatch points either way.
+    constexpr int KB = bwd_points_per_thread(F);
+    constexpr int kBatchPts = kTileThreads * KB;
+    // this thread's points of the batch: row index, coordinates
+    // (coordinates as floats when a thread holds several points -- the double unit coordinate is then rebuilt per
+    // level chunk, 6 registers instead of 12 at the image shape -- and as doubles when it holds one)
+    constexpr bool kKeepUnit = KB * D <= 4;
+    // PIPE: the point's index (the row offset is formed per request: one register per point less while the prologue
+    // batch waits behind the geometry); otherwise the row offset
+    using RowT = std::conditional_t<PIPE, int, int64_t>;
+    RowT rowk[KB];
+    float ck[KB][D];
+    double tu[kKeepUnit ? KB : 1][D];
+    bool livek[KB];
+    float gk[KB][kLv * F];
+    // PIPE (2D): the next level chunk's gradient pieces go to thread-private shared-memory slots with cp.async while
+    // the current chunk is reduced and accumulated, and reach gk with one LDS each -- no second set of row registers
+    static_assert(!PIPE || bwd_pipelined(D, F), "the next-chunk slots are laid out for the 2D register batches");
+    constexpr int PC = kLv * F / 4;   // 16-byte pieces per point and level chunk
+    float4* s_next = reinterpret_cast<float4*>(s_dyn + ((s_gS - s_dyn + (DEC ? (ZP ? NW : 1) * L * F : 0) + 3) & ~3));
+    auto request_chunk = [&](int l0) {
+#pragma unroll
+        for (int k = 0; k < KB; ++k)
+#pragma unroll
+            for (int pc = 0; pc < PC; ++pc)
+                cp_async16(s_next + (k * PC + pc) * kTileThreads + threadIdx.x,
+                           grad_out + (int64_t)rowk[k] * L * F + l0 * F + 4 * pc, livek[k] ? 16 : 0);
+        cp_async_commit();
+    };
+    auto load_points = [&](int b0, int b1) {
+#pragma unroll
+        for (int k = 0; k < KB; ++k) {
+            const int j = b0 + k * kTileThreads + threadIdx.x;
+            livek[k] = j < b1;
+            rowk[k] = 0;
+#pragma unroll
+            for (int d = 0; d < D; ++d) ck[k][d] = 0.0f;
+            if (livek[k]) {
+                const int pt = pv.perm ? __ldg(pv.perm + j) : j;
+                rowk[k] = PIPE ? (RowT)pt : (RowT)((int64_t)pt * L * F);
+#pragma unroll
+                for (int d = 0; d < D; ++d) ck[k][d] = __ldg(pv.coords_sorted + (int64_t)j * D + d);
+            }
+            if (kKeepUnit) {
+#pragma unroll
+                for (int d = 0; d < D; ++d) tu[k][d] = unit_coord(ck[k][d]);
+            }
+        }
+    };
+    // PIPE: moves the requested chunk from the thread's slots to gk
+    auto take_chunk = [&]() {
+        cp_async_wait_all();
+#pragma unroll
+        for (int k = 0; k < KB; ++k)
+#pragma unroll
+            for (int pc = 0; pc < PC; ++pc) {
+                const float4 a = s_next[(k * PC + pc) * kTileThreads + threadIdx.x];
+                gk[k][4 * pc] = a.x; gk[k][4 * pc + 1] = a.y; gk[k][4 * pc + 2] = a.z; gk[k][4 * pc + 3] = a.w;
+            }
+    };
+    // the batch's first level chunk: into gk, or (PIPE) into the slots -- registers would spill while the prologue
+    // batch waits behind the tile geometry and the staging
+    auto request_first_chunk = [&](int lrun) {
+        if constexpr (PIPE) {
+            if (lrun > 0) request_chunk(0);
+        } else {
+#pragma unroll
+            for (int k = 0; k < KB; ++k) {
+#pragma unroll
+                for (int e = 0; e < kLv * F; ++e) gk[k][e] = 0.0f;
+                if (livek[k] && lrun > 0) load_row<kLv * F>(grad_out + rowk[k], gk[k]);
+            }
+        }
+    };
+    // 2D: the first register batch is requested before the tile geometry, which then runs under those loads
+    // (2D launches run every level: Lrun == L)
+    if constexpr (PIPE) {
+        load_points(beg, min(end, beg + kBatchPts));
+        request_first_chunk(L);
+    }
+
     for (int e = threadIdx.x; e < nA * C * F; e += kTileThreads) s_A[e] = A[e];
     if (DEC)
         for (int e = threadIdx.x; e < (ZP ? NW : 1) * L * (C * F + F); e += kTileThreads) s_gA[e] = 0.0f;
@@ -721,14 +872,6 @@ latent_bwd_tiled_kernel(const PlanView pv, const float* __restrict__ grad_out, c
     // levels this launch touches: all of them, or the staged prefix rounded up to the level blocking
     const int Lrun = skip_direct ? min(L, ((__popc(tg.staged) + kLv - 1) / kLv) * kLv) : L;
 
-    // Points per thread held in registers for a whole batch: each 16-byte piece of a gradient row is read ONCE, its
-    // levels' maxima (the fixed-point scales) are reduced from the registers, and after one barrier the same registers
-    // feed the accumulation -- no separate max pass over the rows (round 1: a second, latency-bound read of every row).
-    // A tile with more points than one register batch (uneven sample sets; the test suite's clustered case) runs the
-    // max pass of round 1 over up to kBatch points first and then several register batches into the SAME accumulators:
-    // one zero-fill and one flush per kBatch points either way.
-    constexpr int KB = (F == 1) ? 3 : ((F == 2) ? 2 : 1);
-    constexpr int kBatchPts = kTileThreads * KB;
     for (int s0 = beg; s0 < end; s0 += kBatch) {
         const int s1 = min(end, s0 + kBatch);
         // (the 3D staged-prefix launches always take this form: their tiles average 128 samples around a batch of 128,
@@ -801,54 +944,34 @@ latent_bwd_tiled_kernel(const PlanView pv, const float* __restrict__ grad_out, c
         const bool own_max = !level_max && !multi;   // the chunk loop reduces the maxima itself (one register batch)
       for (int b0 = s0; b0 < s1; b0 += kBatchPts) {
         const int b1 = min(s1, b0 + kBatchPts);
-        // this thread's points of the batch: row index, coordinates
-        // (coordinates as floats when a thread holds several points -- the double unit coordinate is then rebuilt per
-        // level chunk, 6 registers instead of 12 at the image shape -- and as doubles when it holds one)
-        constexpr bool kKeepUnit = KB * D <= 4;
-        int64_t rowk[KB];
-        float ck[KB][D];
-        double tu[kKeepUnit ? KB : 1][D];
-        bool livek[KB];
-#pragma unroll
-        for (int k = 0; k < KB; ++k) {
-            const int j = b0 + k * kTileThreads + threadIdx.x;
-            livek[k] = j < b1;
-            rowk[k] = 0;
-#pragma unroll
-            for (int d = 0; d < D; ++d) ck[k][d] = 0.0f;
-            if (livek[k]) {
-                rowk[k] = (int64_t)(pv.perm ? __ldg(pv.perm + j) : j) * L * F;
-#pragma unroll
-                for (int d = 0; d < D; ++d) ck[k][d] = __ldg(pv.coords_sorted + (int64_t)j * D + d);
-            }
-            if (kKeepUnit) {
-#pragma unroll
-                for (int d = 0; d < D; ++d) tu[k][d] = unit_coord(ck[k][d]);
-            }
-        }
+        const bool prologue_batch = PIPE && b0 == beg;   // loaded before the tile geometry
+        if (!prologue_batch) load_points(b0, b1);
         // latents for the decoder gradients (ZP: per-point z; SG: q[node] at flush), staged once, behind the loads above
         if (DEC && !staged_lat) {
             stage_nodes<D, C>(tg, pv.node_tab + (size_t)tile * pv.node_stride, latents, round_flag, s_lat);
             staged_lat = true;
         }
         // the first chunk's gradient pieces are requested before the barrier, every later chunk's while the previous one
-        // is being accumulated (SHACIRA_BWD_PREFETCH: one more set of row registers)
-        float gk[KB][kLv * F];
-#pragma unroll
-        for (int k = 0; k < KB; ++k) {
-#pragma unroll
-            for (int e = 0; e < kLv * F; ++e) gk[k][e] = 0.0f;
-            if (livek[k] && Lrun > 0) load_row<kLv * F>(grad_out + rowk[k], gk[k]);
+        // is being accumulated
+        if (!prologue_batch) request_first_chunk(Lrun);
+        if constexpr (PIPE) {
+            // chunk 0 to gk; chunk 1 is an L2 hit (the first request fetched its 64-byte block) and arrives under chunk 0
+            take_chunk();
+            if (Lrun > kLv) request_chunk(kLv);
         }
         __syncthreads();
         for (int l0 = 0; l0 < Lrun; l0 += kLv) {
-#if !SHACIRA_BWD_PREFETCH
             if (l0 > 0) {
+                if constexpr (PIPE) {
+                    // this chunk's pieces are in the thread's slots; the next chunk's are requested into the same slots
+                    take_chunk();
+                    if (l0 + kLv < Lrun) request_chunk(l0 + kLv);
+                } else {
 #pragma unroll
-                for (int k = 0; k < KB; ++k)
-                    if (livek[k]) load_row<kLv * F>(grad_out + rowk[k] + l0 * F, gk[k]);
+                    for (int k = 0; k < KB; ++k)
+                        if (livek[k]) load_row<kLv * F>(grad_out + rowk[k] + l0 * F, gk[k]);
+                }
             }
-#endif
             if (own_max) {
                 // maxima of what this chunk of levels will accumulate, over the batch: REDUX over the warp, one shared
                 // atomicMax per warp and level; NaN propagates (nan_max; its bit pattern compares above +Inf)
@@ -878,15 +1001,6 @@ latent_bwd_tiled_kernel(const PlanView pv, const float* __restrict__ grad_out, c
                 }
                 __syncthreads();
             }
-#if SHACIRA_BWD_PREFETCH
-            float gn[KB][kLv * F];
-#pragma unroll
-            for (int k = 0; k < KB; ++k) {
-#pragma unroll
-                for (int e = 0; e < kLv * F; ++e) gn[k][e] = 0.0f;
-                if (livek[k] && l0 + kLv < Lrun) load_row<kLv * F>(grad_out + rowk[k] + (l0 + kLv) * F, gn[k]);
-            }
-#endif
             float accS[ZP ? kLv * F : 1], accA[ZP ? kLv * C * F : 1];
             if (ZP) {
 #pragma unroll
@@ -1072,12 +1186,6 @@ latent_bwd_tiled_kernel(const PlanView pv, const float* __restrict__ grad_out, c
                     if (lane == 0) s_gA[(warp * L + l0) * C * F + e] += v;  // e = (q*C + ch)*F + jf
                 }
             }
-#if SHACIRA_BWD_PREFETCH
-#pragma unroll
-            for (int k = 0; k < KB; ++k)
-#pragma unroll
-                for (int e = 0; e < kLv * F; ++e) gk[k][e] = gn[k][e];
-#endif
         }
       }   // register batches of this span
         if (threadIdx.x < L) {
