@@ -407,6 +407,35 @@ int shacira_prune_samples(int32_t res, const float* jitter, float* samples, shac
 int shacira_prune_update(int64_t cells, const float* density, float decay, float min_density, float* occupancy,
                          uint8_t* mask, shacira_stream_t stream);
 
+/* ---- NeRF decoder heads on the tensor cores (NeuralRadianceField.rgba, wisp/models/nefs/nerf.py:218-233) ---- */
+/* decoder_density: in_dim -> hidden_dim -> 16, decoder_color: (16 + emb_dim) -> hidden_dim -> hidden_dim -> 3. With b()
+ * = round to nearest even bf16, fp32 products and biases (DESIGN section 9):
+ *   h1 = relu(b(X) b(W1)^T + b1)   d = b(h1) b(W2)^T + b2   density = relu(d[:, 0])
+ *   u = [b(d), b(vemb[ridx])]      h2 = relu(u b(W3)^T + b3)   h3 = relu(b(h2) b(W4)^T + b4)
+ *   rgb = sigmoid(b(h3) b(W5)^T + b5)
+ * feats [num_samples, in_dim] fp32 (16-byte aligned), vemb [num_rays, emb_dim] one row per ray, ridx [num_samples]
+ * int32; a ridx outside [0, num_rays) takes a zero embedding. params = {W1, b1, W2, b2, W3, b3, W4, b4, W5, b5}, fp32 in
+ * torch.nn.Linear layout ([out, in] and [out]). Supported: in_dim 64 or 96, hidden_dim 128, emb_dim 0 .. 32; anything
+ * else is SHACIRA_ERR_UNSUPPORTED. num_samples = 0 is a successful no-op. No host synchronisation (graph capturable).
+ * forward: density [num_samples], rgb [num_samples, 3]. density_only != 0 runs the density head alone: vemb, ridx,
+ * rgb and params[4..9] are not read and may be NULL. */
+int shacira_nerf_heads_forward(const float* feats, int64_t num_samples, int32_t in_dim, int32_t hidden_dim,
+                               const float* vemb, int32_t num_rays, int32_t emb_dim, const int32_t* ridx,
+                               const float* const* params, int32_t density_only, float* density, float* rgb,
+                               shacira_stream_t stream);
+/* backward: recomputes the forward from feats, then writes grad_feats [num_samples, in_dim] (16-byte aligned) and the
+ * ten parameter gradients grad_params (same order and shapes as params; overwritten, not accumulated) from
+ * grad_density [num_samples] and grad_rgb [num_samples, 3]. Every gradient operand of a product is rounded with b();
+ * the weight gradients are b(g)^T b(activation) over all samples, the bias gradients fp32 sums of the gradient. Both
+ * are summed in a fixed order (no float atomics): repeated calls are bit-identical. No gradient reaches vemb.
+ * workspace: device memory of at least shacira_nerf_heads_workspace_bytes(in_dim) bytes (per-CTA partial sums). */
+int64_t shacira_nerf_heads_workspace_bytes(int32_t in_dim);
+int shacira_nerf_heads_backward(const float* feats, int64_t num_samples, int32_t in_dim, int32_t hidden_dim,
+                                const float* vemb, int32_t num_rays, int32_t emb_dim, const int32_t* ridx,
+                                const float* const* params, const float* grad_density, const float* grad_rgb,
+                                float* grad_feats, float* const* grad_params, void* workspace, int64_t workspace_bytes,
+                                shacira_stream_t stream);
+
 /* ---- latent bitstream (host side) ---------------------------------------------------- */
 /* Static arithmetic coder over dense symbol ranks 0..num_symbols-1 with 16-bit cumulative
  * frequencies cdf[num_symbols+1] (cdf[0] = 0, strictly increasing, cdf[num_symbols] = 65536).

@@ -112,6 +112,9 @@ SIGNATURES = {
     "shacira_raytrace_dense_fill": (ctypes.c_int, [_vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "shacira_prune_samples": (ctypes.c_int, [_i32, _vp, _vp, _vp]),
     "shacira_prune_update": (ctypes.c_int, [_i64, _vp, ctypes.c_float, ctypes.c_float, _vp, _vp, _vp]),
+    "shacira_nerf_heads_forward": (ctypes.c_int, [_vp, _i64, _i32, _i32, _vp, _i32, _i32, _vp, ctypes.POINTER(_vp), _i32, _vp, _vp, _vp]),
+    "shacira_nerf_heads_workspace_bytes": (_i64, [_i32]),
+    "shacira_nerf_heads_backward": (ctypes.c_int, [_vp, _i64, _i32, _i32, _vp, _i32, _i32, _vp, ctypes.POINTER(_vp), _vp, _vp, _vp, ctypes.POINTER(_vp), _vp, _i64, _vp]),
     "shacira_ac_encode": (_i64, [_vp, _i64, _vp, _i32, _vp, _i64]),
     "shacira_ac_decode": (ctypes.c_int, [_vp, _i64, _vp, _i32, _vp, _i64]),
     "shacira_latent_step_host": (ctypes.c_int, [_i32, _vp, _i64, _vp, _i64, _c_int32_p, _c_int32_p, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp]),

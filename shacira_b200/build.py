@@ -10,7 +10,7 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libshacira_b200.so")
-SOURCES = ["capi.cu", "tiled_capi.cu", "grid3d_capi.cu", "session_capi.cu", "peer_capi.cu"]
+SOURCES = ["capi.cu", "tiled_capi.cu", "grid3d_capi.cu", "session_capi.cu", "peer_capi.cu", "nerf_heads_capi.cu"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O3",
